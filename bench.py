@@ -54,7 +54,38 @@ def parse():
     ap.add_argument("--groups", type=int, default=-1, help="wave scheduler only: worker streams per GPU (-1: library default)")
     ap.add_argument("--slots", type=int, default=-1, help="wave scheduler only: pairs advanced in lock-step per stream (-1: library default)")
     ap.add_argument("--spec", type=int, default=-1, help="wave scheduler only: speculation width in rotation nodes (-1: library default)")
-    return ap.parse_args()
+    ap.add_argument("--dump-outputs", metavar="DIR", help="write the registrations of rank 0's last timed step as DIR/<name>.npy (see dump_outputs)")
+    args = ap.parse_args()
+    if args.steps < 1:
+        ap.error("--steps must be at least 1")
+    if args.dump_outputs and args.impl == "reference":
+        ap.error("--dump-outputs writes what the GPU arm computed; it does not apply to --impl reference")
+    return args
+
+
+DUMP_ROWS = 100000   # 172 B per registration: two dumped legs stay under 64 MB
+
+
+def dump_outputs(out_dir, results, prefix=""):
+    """The arrays a caller receives from one timed step, one row per registration: R (n,3,3), t (n,3), opt_error (n,),
+    opt_comp (n,), status (n,), the search counters 0-5 of goicp_result (n,6) and index (n,), the row's position in the step.  Counters 6-7
+    (launches, speculative re-runs) describe the schedule, not the result, and are left out.  A step of more than DUMP_ROWS
+    registrations is written as a fixed, seeded sample of them.  The inputs are seeded too, so two builds run with the same
+    arguments can be compared file for file."""
+    idx = np.arange(len(results))
+    if len(idx) > DUMP_ROWS:
+        idx = np.sort(np.random.default_rng(0).choice(len(idx), DUMP_ROWS, replace=False))
+    rows = [results[i] for i in idx]
+    os.makedirs(out_dir, exist_ok=True)
+    arrays = {"R": np.array([r["R"] for r in rows], np.float64).reshape(-1, 3, 3),
+              "t": np.array([r["t"] for r in rows], np.float64).reshape(-1, 3),
+              "opt_error": np.array([r["optError"] for r in rows], np.float32),
+              "opt_comp": np.array([r["optComp"] for r in rows], np.float64),
+              "status": np.array([r["status"] for r in rows], np.float64),
+              "counters": np.array([list(r["counters"])[:6] for r in rows], np.float64).reshape(-1, 6),
+              "index": idx.astype(np.float64)}
+    for name, a in arrays.items():
+        np.save(os.path.join(out_dir, prefix + name + ".npy"), a)
 
 
 def config_dict(args):
@@ -224,7 +255,7 @@ def deep_arm(args, g, synth, rank, world, local):
     sampler = ClockSampler(local)
     if rank == 0:
         sampler.start()
-    rows = []
+    rows, last = [], []
     for name, m, d, nd, params, cl in cases:
         reg = g.GoICP(m, d, params, device=local, **cl)
         reg.BuildDT(); reg.set_nd(nd)
@@ -245,6 +276,7 @@ def deep_arm(args, g, synth, rank, world, local):
                 dist.barrier()
             torch.cuda.synchronize(dev)
             t0 = time.perf_counter(); r = reg.Register(); torch.cuda.synchronize(dev); ts.append(1e3 * (time.perf_counter() - t0))
+        last.append(r)
         sig = torch.tensor([sum(ts), r["optError"]] + [float(v) for v in r["counters"][:6]], dtype=torch.float64, device=dev)
         same = True
         if world > 1:
@@ -260,6 +292,8 @@ def deep_arm(args, g, synth, rank, world, local):
                      "exact_order_1gpu": None if exact is None else {"ms": t_exact, "opt_error": exact["optError"], "rotation_pops": int(exact["counters"][3]), "inner_calls": int(exact["counters"][0])}})
         del reg
     sampler.stop_flag = True
+    if args.dump_outputs and rank == 0:
+        dump_outputs(args.dump_outputs, last)
     if rank == 0:
         h = rows[0]
         print(json.dumps({"metric": METRIC, "value": h["value"], "unit": UNIT, "n_gpus": world, "steps": args.steps, "warmup": args.warmup, "ms_per_step": h["ms_per_registration"],
@@ -353,6 +387,9 @@ def main():
         e2e_ms += 1e3 * (time.perf_counter() - t1); e2e_evals += float(sum(r.counters[2] * p["nd"] for r, p in zip(r2, pairs)))
     barrier()
     sampler.stop_flag = True
+    if args.dump_outputs and rank == 0:
+        dump_outputs(args.dump_outputs, res)
+        dump_outputs(args.dump_outputs, [g._result_dict(r) for r in r2], prefix="e2e_")
     h2d = sum(p[k].nbytes for p in pairs for k in ("model_xyz", "data_xyz", "model_c", "data_c")) + (sum(p["model_fpfh"].nbytes + p["data_fpfh"].nbytes for p in pairs) if args.fpfh else 0)
     d2h = len(pairs) * 208
 

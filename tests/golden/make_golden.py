@@ -151,6 +151,32 @@ def make_inclusion():
     np.savez_compressed(os.path.join(OUT, "rand_inclusion.npz"), **fx)
 
 
+def make_inner(kind="ref"):
+    """function-level values on cavity pair 2 (shipped config): weights, maxRotDis, DT3D::Distance of 2 000 seeded queries,
+    InnerBnB of 6 seeded rotations at levels -1 and 1 against optError 30, and one ICP from the identity.  The inputs are the ones
+    tests/test_oracle_golden.py::test_port_vs_reference_inner_calls always used, and they are stored beside the values.  `kind`
+    names the implementation that produced them; it is stored as `source`."""
+    print("pair2_inner", kind)
+    sys.path.insert(0, os.path.join(ROOT, "tests"))
+    from conftest import rand_rot
+    z = np.load(os.path.join(OUT, "pair2.npz"))
+    o = po.Oracle(kind, z["model_xyz"], z["data_xyz"], po.shipped_config(), model_c=z["model_c"], data_c=z["data_c"],
+                  model_fpfh=z["model_fpfh"], data_fpfh=z["data_fpfh"])
+    o.build_dt(); o.set_nd(int(z["nd"])); o.initialize()
+    rng = np.random.default_rng(1)
+    q = rng.uniform(-1.5, 1.5, (2000, 3))
+    Rs = np.stack([rand_rot(rng) for _ in range(6)])
+    inner = [[o.inner_bnb(R, level, 30.0) for level in (-1, 1)] for R in Rs]
+    e, R, t, corr = o.icp(np.eye(3), np.zeros(3))
+    fx = dict(source=np.array(kind), weights=o.weights(), maxrotdis=o.maxrotdis(), q=q, dist=o.dt_distance(q)[0], R=Rs,
+              levels=np.array([-1, 1], np.int32), inner_opt_error=np.float32(30.0),
+              inner_err=np.array([[v[0] for v in row] for row in inner], np.float32),
+              inner_tnode=np.array([[v[1] for v in row] for row in inner], np.float32),
+              icp_err=np.float32(e), icp_R=R, icp_t=t, icp_corr=corr)
+    o.close()
+    np.savez_compressed(os.path.join(OUT, "pair2_inner.npz"), **fx)
+
+
 def make_deep_small():
     """BASELINE config 4 (synthetic deep search) at a size the reference finishes in minutes: target 20 000 points on the bumpy
     sphere, source 2 000 of them moved by a random rigid motion + noise (go-icp-protein-cavities_b200/synth.py:deep_pair, seed 1241),
@@ -168,12 +194,14 @@ def make_deep_small():
 
 if __name__ == "__main__":
     po.build("ref")
-    which = sys.argv[1:] or ["pair1", "pair2", "rand", "bunny", "inclusion"]
+    which = sys.argv[1:] or ["pair1", "pair2", "inner", "rand", "bunny", "inclusion"]
     with tempfile.TemporaryDirectory() as tmp:
         if "pair1" in which:
             make_pair("pair1", "1eq2_6", "2x86_3", 238, tmp, fpfh_variant=True)
         if "pair2" in which:
             make_pair("pair2", "4imo_2", "2ktd_1", 247, tmp)
+        if "inner" in which:
+            make_inner()
         if "rand" in which:
             make_demo("rand", "model_rand.txt", "data_rand.txt", 100, 0.1, [64, 300])
         if "bunny" in which:
