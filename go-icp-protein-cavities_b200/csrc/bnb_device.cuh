@@ -209,12 +209,11 @@ struct CancelSh { const volatile unsigned* word; unsigned gen; int flag; };
 // One request = one InnerBnB call, or (level >= GOICP_REQ_BOTH) the upper- and the lower-bound call of one rotation cube.
 // Called by every thread of the CTA; `pr` and `s_out` live in shared memory; the result is left in `s_out` (thread 0 wrote it;
 // a __syncthreads / __syncwarp of warp 0 is needed before other threads read it).  `s_gbar` is an mbarrier initialised once by the
-// kernel (GS only).  dstat: device counters [0] busy cycles [1] pops [2] corner misses [3] calls.
+// kernel (GS only).  `ctr` collects the device counters.
 template <bool EXACT, bool SMEM, bool GS, bool CT, bool CANCEL>
 __device__ __forceinline__ void inner_call(const PairDev* __restrict__ pairs, const InnerProb& pr, InnerOut& s_out, unsigned long long& s_gbar, CallCtx& cx, CancelSh& cs,
                                            HeapEnt* __restrict__ heaps, int heapCap, float* gscratch, size_t gstride, int NdP, int NdQ, int useSmem,
-                                           uint4* memoAll, int memoCap, unsigned* genCounter, int gridOff, int S3p) {
-    unsigned long long* dstat = reinterpret_cast<unsigned long long*>(genCounter) + 1;
+                                           uint4* memoAll, int memoCap, DevCounters* ctr, int gridOff, int S3p) {
     extern __shared__ float4 dyn_smem4[];
     __shared__ BnbShared sh;
     __shared__ uint2 s_hkey[HK_SMEM];
@@ -293,7 +292,7 @@ __device__ __forceinline__ void inner_call(const PairDev* __restrict__ pairs, co
         if (tid < 27) sh.cnt[tid] = 0;
         if (tid == 0) {
             sh.status = 0; sh.pops = 1; sh.subcubes = 0; sh.improved = 0;
-            if (cpart == 0) { sh.gen = atomicAdd(genCounter, 1u) + 1u; sh.t0 = clock64(); sh.missTot = 0; }
+            if (cpart == 0) { sh.gen = atomicAdd(&ctr->gen, 1u) + 1u; sh.t0 = clock64(); sh.missTot = 0; }
             sh.nmiss = 0; sh.workCtr = 0; sh.workA = 0;
 #ifdef GOICP_PHASE_TIMING
             if (cpart == 0) for (int k = 0; k < 12; k++) sh.tp[k] = 0;
@@ -732,13 +731,13 @@ __device__ __forceinline__ void inner_call(const PairDev* __restrict__ pairs, co
             } else {
                 s_out.err2 = optT; s_out.pops2 = sh_pops; s_out.subcubes2 = sh_subcubes; s_out.ran2 = 1; s_out.status = sh.status;
             }
-            atomicAdd(dstat + 1, (unsigned long long)sh_pops); atomicAdd(dstat + 3, 1ull);
+            atomicAdd(&ctr->pops, (unsigned long long)sh_pops); atomicAdd(&ctr->calls, 1ull);
         }
         }   // cpart
         if (tid == 0) {
-            atomicAdd(dstat + 0, (unsigned long long)(clock64() - sh.t0)); atomicAdd(dstat + 2, (unsigned long long)sh.missTot);
+            atomicAdd(&ctr->callCycles, (unsigned long long)(clock64() - sh.t0)); atomicAdd(&ctr->cornerMisses, (unsigned long long)sh.missTot);
 #ifdef GOICP_PHASE_TIMING
-            for (int k = 0; k < 12; k++) atomicAdd(dstat + 8 + k, (unsigned long long)sh.tp[k]);
+            for (int k = 0; k < 12; k++) atomicAdd(&ctr->phaseCycles[k], (unsigned long long)sh.tp[k]);
 #endif
         }
     }

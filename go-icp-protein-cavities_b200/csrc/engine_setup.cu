@@ -70,8 +70,6 @@ goicp_status prepare_problem(Eng* h, Problem& P) {
     return GOICP_OK;
 }
 
-static bool need_corner_terms(const goicp_params& p) { return p.regularization > 0 || p.regularizationNeighbors > 0 || (p.regularizationFPFH > 0 && p.cfpfh != 0); }
-
 // ---- device layout + upload of all problems ----------------------------------------------------------------------
 goicp_status upload_problems(Eng* h) {
     const goicp_params& p = h->params;

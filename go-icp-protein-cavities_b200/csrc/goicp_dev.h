@@ -2,6 +2,7 @@
 // Host code (engine.cu) fills these; kernels only read them (except the marked workspaces).
 // All file:line citations are relative to the reference checkout (guillaumebaldi/Go-ICP-protein-cavities).
 #pragma once
+#include <stddef.h>
 #include <stdint.h>
 
 #define GOICP_MAXROTLEVEL 20               // jly_goicp.h:95
@@ -101,9 +102,10 @@ struct alignas(64) InnerOut {   // one 64-byte record: it leaves the SM as a sin
 
 struct alignas(16) HeapEnt { float lb, w, x, y, z, pad0, pad1, pad2; };   // TRANSNODE without ub (never read, jly_goicp.h:75-87)
 
+enum IcpMode { ICP_REFINE = 0, ICP_INIT_ERROR = 1, ICP_COMPAT = 2 };   // ICP + re-score (:102), error at the identity (:601-627), updateCompatibilities (:933)
 struct IcpState {           // one GoICP::ICP call (jly_goicp.cpp:102) in flight
     int pair;
-    int mode;               // 0 ICP + re-score, 1 initial error at identity (:601-627), 2 updateCompatibilities (:933)
+    int mode;               // IcpMode
     double R[9], t[3];
     double mu_m[3], mu_d[3];  // never reset between iterations (jly_icp3d.hpp:221-222, SURVEY Q4)
     float err;              // previous err (-1 at start)
@@ -114,7 +116,25 @@ struct IcpState {           // one GoICP::ICP call (jly_goicp.cpp:102) in flight
     float error;
     int incomp;             // countCompatibilities over the correspondences
     float fpfh;
-    int compat_pose;        // checkCompatibility count at the pose (mode 2)
+    int compat_pose;        // checkCompatibility count at the pose (ICP_COMPAT)
 };
 
 struct WaveCube { float x, y, z, w; int rot; };   // a child translation cube to evaluate under rotation `rot`
+
+// Counters of one handle's kernels: the corner memo's generation word, then statistics the host reads and clears after each search
+struct DevCounters {
+    unsigned gen;   // bumped per call: tags the call's entries in the corner memo
+    unsigned long long callCycles, pops, cornerMisses, calls;   // all calls: CTA cycles inside calls, translation-queue pops, corner evaluations the memo missed, calls
+    unsigned long long idleCycles, unused, icpRequests, ctaCycles;   // search kernel: CTA cycles scheduling / waiting / idle, (none), ICP requests, CTA cycles in total
+    unsigned long long phaseCycles[12];   // per-phase cycles of a pop (built with -DGOICP_PHASE_TIMING)
+};
+static_assert(offsetof(DevCounters, gen) == 0, "");
+static_assert(offsetof(DevCounters, callCycles) == 8, "");
+static_assert(offsetof(DevCounters, pops) == 16, "");
+static_assert(offsetof(DevCounters, cornerMisses) == 24, "");
+static_assert(offsetof(DevCounters, calls) == 32, "");
+static_assert(offsetof(DevCounters, idleCycles) == 40, "");
+static_assert(offsetof(DevCounters, unused) == 48, "");
+static_assert(offsetof(DevCounters, icpRequests) == 56, "");
+static_assert(offsetof(DevCounters, ctaCycles) == 64, "");
+static_assert(offsetof(DevCounters, phaseCycles) == 72 && sizeof(DevCounters) == 168, "");

@@ -16,8 +16,8 @@ __device__ __forceinline__ void icp_begin_part(const PairDev& P, IcpState& st) {
     __syncthreads();
     int bad = 0;
     for (int i = threadIdx.x; i < Nd; i += blockDim.x) {
-        if (st.mode == 0) { P.nn[i] = GOICP_NN_EMPTY; P.order[i] = i; }   // modes 1/2 may share a launch with a mode-0 state of the same pair
-        if (st.mode == 2) {
+        if (st.mode == ICP_REFINE) { P.nn[i] = GOICP_NN_EMPTY; P.order[i] = i; }   // ICP_INIT_ERROR / ICP_COMPAT may share a launch with an ICP_REFINE state of the same pair
+        if (st.mode == ICP_COMPAT) {
             const double x0 = P.dx[i], y0 = P.dy[i], z0 = P.dz[i];
             const float x = (float)(st.R[0] * x0 + st.R[1] * y0 + st.R[2] * z0 + st.t[0]);
             const float y = (float)(st.R[3] * x0 + st.R[4] * y0 + st.R[5] * z0 + st.t[1]);
@@ -26,7 +26,7 @@ __device__ __forceinline__ void icp_begin_part(const PairDev& P, IcpState& st) {
             bad += ((P.g.cmask[cell] >> P.dprop[i]) & 1u) ? 0 : 1;
         }
     }
-    if (st.mode == 2) {
+    if (st.mode == ICP_COMPAT) {
         bad = warp_sum_i(bad);
         if ((threadIdx.x & 31) == 0) atomicAdd(&s_cnt, bad);
         __syncthreads();
@@ -222,7 +222,7 @@ __device__ __forceinline__ bool icp_update_part(const PairDev& P, IcpState& st, 
 // ---- scoring: initial error at identity (jly_goicp.cpp:601-627) or the DT re-score of GoICP::ICP (:117-175) ---------
 __device__ __forceinline__ void icp_score_part(const PairDev& P, IcpState& st) {
     const int Nd = P.Nd, tid = threadIdx.x, lane = tid & 31, warp = tid >> 5;
-    float* val = P.scratch + (st.mode == 1 ? 7 * Nd : 0);   // Nd: per data index; mode 1 may run beside a mode-0 state whose update uses [0, 7 Nd)
+    float* val = P.scratch + (st.mode == ICP_INIT_ERROR ? 7 * Nd : 0);   // Nd: per data index; ICP_INIT_ERROR may run beside an ICP_REFINE state whose update uses [0, 7 Nd)
     float* fd = P.scratch + Nd;        // Nd: per position of `order`
     __shared__ int s_bad, s_nb;
     __shared__ float s_geom, s_fpfh, s_trim;
@@ -231,7 +231,7 @@ __device__ __forceinline__ void icp_score_part(const PairDev& P, IcpState& st) {
     int bad = 0, nb = 0;
     for (int i = tid; i < Nd; i += blockDim.x) {
         float x, y, z;
-        if (st.mode == 1) { x = P.dx[i]; y = P.dy[i]; z = P.dz[i]; }
+        if (st.mode == ICP_INIT_ERROR) { x = P.dx[i]; y = P.dy[i]; z = P.dz[i]; }
         else {
             const double x0 = P.dx[i], y0 = P.dy[i], z0 = P.dz[i];
             x = (float)(st.R[0] * x0 + st.R[1] * y0 + st.R[2] * z0 + st.t[0]);       // double expr -> float store :120-122
@@ -239,8 +239,8 @@ __device__ __forceinline__ void icp_score_part(const PairDev& P, IcpState& st) {
             z = (float)(st.R[6] * x0 + st.R[7] * y0 + st.R[8] * z0 + st.t[2]);
         }
         const float dt = dt_distance(P.g, P.g.dist, x, y, z);
-        val[i] = (st.mode == 0 && P.doTrim) ? dt : P.weights[i] * dt;                // :135: no weight when trimming
-        if (st.mode == 0) {
+        val[i] = (st.mode == ICP_REFINE && P.doTrim) ? dt : P.weights[i] * dt;                // :135: no weight when trimming
+        if (st.mode == ICP_REFINE) {
             const int idd = P.order[i];
             const int idm = (int)(P.nn[idd] & 0xFFFFFFFFu);
             if (P.cfpfh != 0) {   // computeFPFHDifference(true, i) :1625-1641
@@ -252,7 +252,7 @@ __device__ __forceinline__ void icp_score_part(const PairDev& P, IcpState& st) {
             if (P.use_nb) nb += abs(P.nbD[idd] - P.nbM[idm]);                  // compareNeighbors(true) :1250-1288
         }
     }
-    if (st.mode == 0) { bad = warp_sum_i(bad); nb = warp_sum_i(nb); if (lane == 0) { atomicAdd(&s_bad, bad); atomicAdd(&s_nb, nb); } }
+    if (st.mode == ICP_REFINE) { bad = warp_sum_i(bad); nb = warp_sum_i(nb); if (lane == 0) { atomicAdd(&s_bad, bad); atomicAdd(&s_nb, nb); } }
     __syncthreads();
     if (!P.doTrim) {
         if (tid == 0) {   // sequential float sum in index order
@@ -263,10 +263,10 @@ __device__ __forceinline__ void icp_score_part(const PairDev& P, IcpState& st) {
         }
     } else if (warp == 0) {
         float su, sl;
-        warp_trimmed_sums(val, Nd, P.inlierNum, lane, (st.mode == 0) ? 2 : P.norm, 0.f, &su, &sl);   // :171-174 always squares
+        warp_trimmed_sums(val, Nd, P.inlierNum, lane, (st.mode == ICP_REFINE) ? 2 : P.norm, 0.f, &su, &sl);   // :171-174 always squares
         if (lane == 0) s_trim = su;
     }
-    if (st.mode == 0 && P.cfpfh != 0 && tid == 32) {
+    if (st.mode == ICP_REFINE && P.cfpfh != 0 && tid == 32) {
         float f = 0.f;
         for (int i = 0; i < Nd; ++i) f = f + fd[i];
         s_fpfh = f / (float)Nd;                                                      // :147
@@ -274,7 +274,7 @@ __device__ __forceinline__ void icp_score_part(const PairDev& P, IcpState& st) {
     __syncthreads();
     if (tid == 0) {
         float error = s_geom;
-        if (st.mode == 0) {
+        if (st.mode == ICP_REFINE) {
             if (P.use_nb) error = error + P.regN * (float)(s_nb * s_nb);              // :149-153
             if (P.use_reg) error = error + P.reg * (float)(s_bad * s_bad);            // :154-159
             if (P.regF > 0.f) error = error + P.regF * (s_fpfh * s_fpfh);             // :160-163
@@ -305,8 +305,8 @@ __device__ __forceinline__ void icp_fused_body(const PairDev* __restrict__ pairs
     __syncthreads();
     // the state goes back to (possibly mapped host) memory; the system fence orders it before the completion record that thread 0
     // writes afterwards -- a host that sees the record must see the results
-    if (st.mode == 2) { if (tid == 0) { *gstate = st; __threadfence_system(); } return; }
-    if (st.mode == 0) {
+    if (st.mode == ICP_COMPAT) { if (tid == 0) { *gstate = st; __threadfence_system(); } return; }
+    if (st.mode == ICP_REFINE) {
         for (;;) {
             const float r00 = (float)st.R[0], r01 = (float)st.R[1], r02 = (float)st.R[2], r10 = (float)st.R[3], r11 = (float)st.R[4],
                         r12 = (float)st.R[5], r20 = (float)st.R[6], r21 = (float)st.R[7], r22 = (float)st.R[8];

@@ -9,7 +9,7 @@
 //                     fork's incompatibility / c-FPFH / neighbour-count terms the per-call memo does not hold.
 //                     EXACT=true reproduces the reference's sequential float sums bit for bit (16 independent FADD
 //                     chains on 16 lanes of one warp), EXACT=false uses warp-shuffle tree sums.
-//                     One launch per wave of calls (the wave scheduler of engine.cu); the device-resident search (k_search.cu)
+//                     One launch per wave of calls (the wave schedulers of engine_search.cu); the device-resident search (k_search.cu)
 //                     runs the same call code (bnb_device.cuh) inside its own kernel.
 //  eval_bounds_kernel flat wave: one warp per (rotation cube, translation sub-cube), leaf-level (ub, lb) only.
 //
@@ -40,8 +40,7 @@ __global__ void __launch_bounds__(BNB_MAX_THREADS, GOICP_BNB_MIN_CTAS)
 inner_bnb_kernel(const PairDev* __restrict__ pairs, const InnerProb* probs, InnerOut* outs,
                  int nprob, int* __restrict__ counter, HeapEnt* __restrict__ heaps, int heapCap,
                  float* gscratch, size_t gstride, int NdP, int NdQ, int useSmem,
-                 uint4* memoAll, int memoCap, unsigned* genCounter, int gridOff, int S3p) {
-    unsigned long long* dstat = reinterpret_cast<unsigned long long*>(genCounter) + 1;   // [0] busy cycles [1] pops [2] corner misses [3] calls [4] poll cycles
+                 uint4* memoAll, int memoCap, DevCounters* ctr, int gridOff, int S3p) {
     extern __shared__ float4 dyn_smem4[];
     __shared__ InnerProb s_pr;
     __shared__ InnerOut s_out;
@@ -68,7 +67,7 @@ inner_bnb_kernel(const PairDev* __restrict__ pairs, const InnerProb* probs, Inne
         __syncthreads();
         const int p = shk.prob;
         const InnerProb& pr = s_pr;   // (stays in shared memory: R is only read while staging)
-        inner_call<EXACT, SMEM, GS, CT, false>(pairs, pr, s_out, s_gbar, cx, s_cancel, heaps, heapCap, gscratch, gstride, NdP, NdQ, useSmem, memoAll, memoCap, genCounter, gridOff, S3p);
+        inner_call<EXACT, SMEM, GS, CT, false>(pairs, pr, s_out, s_gbar, cx, s_cancel, heaps, heapCap, gscratch, gstride, NdP, NdQ, useSmem, memoAll, memoCap, ctr, gridOff, S3p);
         if (warp == 0) {   // the record leaves the SM as ONE coalesced 64-byte store (it may live in mapped host memory)
             __syncwarp();
             InnerOut* dst = outs + p;
@@ -192,7 +191,7 @@ size_t goicp_bnb_smem_floats(int NdP, int NdQ, bool exact, bool needMd, bool nee
     return n > 3 * 512 ? n : 3 * 512;   // an ICP request tiles the model cloud through the same region (icp_device.cuh NN_TILE)
 }
 
-typedef void (*bnb_kernel_t)(const PairDev*, const InnerProb*, InnerOut*, int, int*, HeapEnt*, int, float*, size_t, int, int, int, uint4*, int, unsigned*, int, int);
+typedef void (*bnb_kernel_t)(const PairDev*, const InnerProb*, InnerOut*, int, int*, HeapEnt*, int, float*, size_t, int, int, int, uint4*, int, DevCounters*, int, int);
 template <bool SMEM, bool GS, bool CT>
 static bnb_kernel_t bnb_kernel_sel(int exact) { return exact ? inner_bnb_kernel<true, SMEM, GS, CT> : inner_bnb_kernel<false, SMEM, GS, CT>; }
 // smem: 0 staging arrays in a global slab, 1 in shared memory, 2 shared memory incl. the DT volume; ct: generic corner terms
@@ -216,14 +215,14 @@ static cudaError_t bnb_attr(int exact, int smem, int ct) {
 
 cudaError_t goicp_launch_inner_bnb(const PairDev* pairs, const InnerProb* probs, InnerOut* outs, int nprob, int* counter,
                                    HeapEnt* heaps, int heapCap, int maxCtas, float* gscratch, size_t gstride,
-                                   int NdP, int NdQ, size_t smemBytes, int useSmem, int gridOff, int S3p, int exact, int ct, int threads, void* memo, int memoCap, unsigned* genCounter, cudaStream_t st, int* ctasLaunched) {
+                                   int NdP, int NdQ, size_t smemBytes, int useSmem, int gridOff, int S3p, int exact, int ct, int threads, void* memo, int memoCap, DevCounters* ctr, cudaStream_t st, int* ctasLaunched) {
     if (nprob <= 0) { if (ctasLaunched) *ctasLaunched = 0; return cudaSuccess; }
     const size_t smem = useSmem ? smemBytes : 0;
     cudaError_t e = bnb_attr(exact, useSmem, ct);
     if (e != cudaSuccess) return e;
     int grid = nprob < maxCtas ? nprob : maxCtas;
     if (ctasLaunched) *ctasLaunched = grid;
-    bnb_kernel(exact, useSmem, ct)<<<grid, threads, smem, st>>>(pairs, probs, outs, nprob, counter, heaps, heapCap, gscratch, gstride, NdP, NdQ, useSmem, (uint4*)memo, memoCap, genCounter, gridOff, S3p);
+    bnb_kernel(exact, useSmem, ct)<<<grid, threads, smem, st>>>(pairs, probs, outs, nprob, counter, heaps, heapCap, gscratch, gstride, NdP, NdQ, useSmem, (uint4*)memo, memoCap, ctr, gridOff, S3p);
     return cudaGetLastError();
 }
 

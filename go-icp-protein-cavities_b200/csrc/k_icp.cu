@@ -21,7 +21,7 @@ icp_begin_kernel(const PairDev* __restrict__ pairs, IcpState* __restrict__ state
 __global__ void __launch_bounds__(NN_THREADS)
 icp_nn_kernel(const PairDev* __restrict__ pairs, IcpState* __restrict__ states, int nchunks, int flaggedOnly) {
     const IcpState& st = states[blockIdx.z];
-    if (st.done || st.mode != 0) return;
+    if (st.done || st.mode != ICP_REFINE) return;
     const PairDev& P = pairs[st.pair];
     const int Nd = P.Nd, Nm = P.Nm;
     if ((int)(blockIdx.x * NN_THREADS) >= Nd) return;
@@ -72,7 +72,7 @@ icp_nn_kernel(const PairDev* __restrict__ pairs, IcpState* __restrict__ states, 
 __global__ void __launch_bounds__(128)
 icp_nn_grid_kernel(const PairDev* __restrict__ pairs, IcpState* __restrict__ states, int cubeMax) {
     const IcpState& st = states[blockIdx.y];
-    if (st.done || st.mode != 0) return;
+    if (st.done || st.mode != ICP_REFINE) return;
     const PairDev& P = pairs[st.pair];
     const GridDev& g = P.g;
     const int Nd = P.Nd, S = g.S, lane = threadIdx.x & 31;
@@ -125,14 +125,14 @@ icp_nn_grid_kernel(const PairDev* __restrict__ pairs, IcpState* __restrict__ sta
 __global__ void __launch_bounds__(256)
 icp_update_kernel(const PairDev* __restrict__ pairs, IcpState* __restrict__ states, int rowCap) {
     IcpState& st = states[blockIdx.x];
-    if (st.done || st.mode != 0) return;
+    if (st.done || st.mode != ICP_REFINE) return;
     extern __shared__ __align__(16) float s_rows[];
     icp_update_part(pairs[st.pair], st, s_rows, rowCap);
 }
 __global__ void __launch_bounds__(256)
 icp_score_kernel(const PairDev* __restrict__ pairs, IcpState* __restrict__ states) {
     IcpState& st = states[blockIdx.x];
-    if (st.mode == 2 || (st.mode == 0 && (!st.done || st.status != 0))) return;
+    if (st.mode == ICP_COMPAT || (st.mode == ICP_REFINE && (!st.done || st.status != 0))) return;
     icp_score_part(pairs[st.pair], st);
 }
 

@@ -284,7 +284,7 @@ __device__ __forceinline__ int owner_serial(Cta& c) {
             os.optT[0] = os.optT[1] = os.optT[2] = 0.0;
             for (int q = 0; q < 2; q++) {
                 IcpState& s = c.icp[q];
-                s.pair = os.pair; s.mode = q == 0 ? 1 : 0;
+                s.pair = os.pair; s.mode = q == 0 ? ICP_INIT_ERROR : ICP_REFINE;
                 for (int k = 0; k < 9; k++) s.R[k] = (k % 4 == 0) ? 1.0 : 0.0;
                 for (int k = 0; k < 3; k++) { s.t[k] = 0.0; s.mu_m[k] = 0.0; s.mu_d[k] = 0.0; }
                 s.err = -1.f; s.iter = 0; s.done = 0; s.status = 0; s.error = 0.f; s.incomp = 0; s.fpfh = 0.f; s.compat_pose = 0;
@@ -321,12 +321,12 @@ __device__ __forceinline__ int owner_serial(Cta& c) {
             if (os.status != 0) { finish_pair(c, 0); os.phase = OW_NONE; break; }
             if (os.heapN == 0) { finish_pair(c, 1); os.phase = OW_NONE; break; }                   // :670-677
             os.quiet++;
-            { const long long tp0 = clock64(); os.par = rq_pop(c.rq, os.heapN); atomicAdd(&A.ctl->dbg[11], (unsigned long long)(clock64() - tp0)); } os.cnt[3]++;
+            { const long long tp0 = clock64(); os.par = rq_pop(c.rq, os.heapN); atomicAdd(&A.ctl->diag[DIAG_POP_CYCLES], (unsigned long long)(clock64() - tp0)); } os.cnt[3]++;
             if ((os.optError - os.par.lb) <= os.SSE) { finish_pair(c, 2); os.phase = OW_NONE; break; }   // :685
             {
                 const uint4 key = node_key(os.par);
                 int g = lookup_group(c, key);   // calls made ahead of time for this node?
-                atomicAdd(&A.ctl->dbg[g >= 0 ? 12 : 13], 1ull);
+                atomicAdd(&A.ctl->diag[g >= 0 ? DIAG_POPS_AHEAD : DIAG_POPS_NOT_AHEAD], 1ull);
                 if (g < 0) {
                     // (no victim: every group has calls running -- they stop at their next pop if abandoned -- or carries the current
                     //  walk stamp, which the pops between two full walks do not advance: age them; the next look-ahead is a full walk)
@@ -348,7 +348,7 @@ __device__ __forceinline__ int owner_serial(Cta& c) {
             }
             const int sidx = 8 * os.par.group + os.j;
             SearchSlot* sl = c.slots + sidx;
-            if (os.pfState[os.j] == SL_DONE) { atomicAdd(&A.ctl->dbg[os.waited ? 15 : 14], 1ull); os.waited = 0; os.waitPolls = 0; } else os.waited = 1;
+            if (os.pfState[os.j] == SL_DONE) { atomicAdd(&A.ctl->diag[os.waited ? DIAG_CHILD_WAITED : DIAG_CHILD_READY], 1ull); os.waited = 0; os.waitPolls = 0; } else os.waited = 1;
             if (os.pfState[os.j] != SL_DONE) {   // not finished when the warp last looked: what is it doing now?
                 const unsigned w = ld_vol(c.st + sidx);
                 const unsigned st = st_of(w);
@@ -396,7 +396,7 @@ __device__ __forceinline__ int owner_serial(Cta& c) {
                     os.optT[0] = (double)(n0 + nw / 2); os.optT[1] = (double)(n1 + nw / 2); os.optT[2] = (double)(n2 + nw / 2);
                     for (int q = 0; q < 2; q++) {   // updateCompatibilities (:791) + ICP(R, t) (:810) at the new incumbent
                         IcpState& s = c.icp[q];
-                        s.pair = os.pair; s.mode = q == 0 ? 2 : 0;
+                        s.pair = os.pair; s.mode = q == 0 ? ICP_COMPAT : ICP_REFINE;
                         for (int k = 0; k < 9; k++) s.R[k] = os.optR[k];
                         for (int k = 0; k < 3; k++) { s.t[k] = os.optT[k]; s.mu_m[k] = 0.0; s.mu_d[k] = 0.0; }
                         s.err = -1.f; s.iter = 0; s.done = 0; s.status = 0; s.error = 0.f; s.incomp = 0; s.fpfh = 0.f; s.compat_pose = 0;
@@ -452,7 +452,7 @@ __device__ __forceinline__ int owner_serial(Cta& c) {
                 while (n > 0) { RNodeD nd = rq_pop(c.rq, n); if (nd.lb < os.optError) { st_node(tmp + m, nd); m++; } else break; }
                 for (int k = 0; k < m; k++) st_node(c.rq + k, ld_node(tmp + k));
                 os.heapN = m;
-                atomicAdd(&A.ctl->dbg[10], (unsigned long long)(clock64() - tp0));
+                atomicAdd(&A.ctl->diag[DIAG_PRUNE_CYCLES], (unsigned long long)(clock64() - tp0));
             }
             { int g; while ((g = alloc_group(c, -1)) < 0) { os.walkStamp++; __nanosleep(200); } os.par.group = g; *reinterpret_cast<uint4*>(os.grpKey[g]) = node_key(os.par); os.grpStamp[g] = os.walkStamp + 1u; }   // the old group drains (calls of the previous incumbent)
             for (int k = 0; k < 8; k++) os.pfState[k] = SL_FREE;
@@ -693,14 +693,14 @@ __device__ __forceinline__ void schedule(Cta& c) {
             if (A.specMax > 0) {
                 int s = -1;
                 const int o = find_help(c, &s);
-                if (o >= 0) { if (lane == 0) { os.action = ACT_CALL; os.actOwner = o; os.actSlot = s; os.actCancel = 1; atomicAdd(&A.ctl->dbg[5], 1ull); } __syncwarp(); return; }
+                if (o >= 0) { if (lane == 0) { os.action = ACT_CALL; os.actOwner = o; os.actSlot = s; os.actCancel = 1; atomicAdd(&A.ctl->diag[DIAG_HELPER_CALLS], 1ull); } __syncwarp(); return; }
             }
             int i = 0;
             if (lane == 0) i = atomicAdd(&A.ctl->nextPair, 1);
             i = __shfl_sync(GOICP_FULL, i, 0);
             if (lane == 0) {
                 if (i < A.npairs) { os.pair = i; os.phase = OW_START; os.manager = 0; st_vol(reinterpret_cast<unsigned*>(&c.hdr->pair), (unsigned)i); atomicAdd(&A.ctl->owners, 1); }
-                else { os.noMorePairs = 1; unsigned long long now; asm volatile("mov.u64 %0, %%globaltimer;" : "=l"(now)); atomicMax(&A.ctl->dbg[8], now - A.ctl->t0ns); atomicCAS(&A.ctl->dbg[9], 0ull, now - A.ctl->t0ns); }
+                else { os.noMorePairs = 1; unsigned long long now; asm volatile("mov.u64 %0, %%globaltimer;" : "=l"(now)); atomicMax(&A.ctl->diag[DIAG_PAIRS_OUT_LAST_NS], now - A.ctl->t0ns); atomicCAS(&A.ctl->diag[DIAG_PAIRS_OUT_FIRST_NS], 0ull, now - A.ctl->t0ns); }
             }
             __syncwarp();
         }
@@ -711,11 +711,11 @@ __device__ __forceinline__ void schedule(Cta& c) {
             // (decided by lane 0 and broadcast: lane 0 rewrites phase and j in owner_serial below, and a lane that evaluated the condition
             //  late would walk into prefetch_group's warp-wide operations alone)
             { int pf = (os.phase == OW_CHILD && os.j < 8) ? 1 : 0; pf = __shfl_sync(GOICP_FULL, pf, 0); if (pf) prefetch_group(c); }
-            if (lane == 0) { rq = owner_serial(c); atomicAdd(&A.ctl->dbg[0], (unsigned long long)(clock64() - tq0)); }
+            if (lane == 0) { rq = owner_serial(c); atomicAdd(&A.ctl->diag[DIAG_OWNER_CYCLES], (unsigned long long)(clock64() - tq0)); }
             rq = __shfl_sync(GOICP_FULL, rq, 0);
             __syncwarp();
             if (rq == RQ_AGAIN) continue;
-            if (rq == RQ_SPAWN) { const long long ts0 = clock64(); spawn_spec(c); if (lane == 0) atomicAdd(&A.ctl->dbg[1], (unsigned long long)(clock64() - ts0)); continue; }
+            if (rq == RQ_SPAWN) { const long long ts0 = clock64(); spawn_spec(c); if (lane == 0) atomicAdd(&A.ctl->diag[DIAG_PUBLISH_CYCLES], (unsigned long long)(clock64() - ts0)); continue; }
             if (rq == RQ_ACTION) {
                 if (os.phase == OW_AFTER_IMPROVE && os.action == ACT_ICP) invalidate_spec(c);   // the incumbent just improved
                 if (os.phase == OW_NONE) {   // the pair is finished
@@ -731,7 +731,7 @@ __device__ __forceinline__ void schedule(Cta& c) {
             if (rq == RQ_WAIT) {   // manager: a helper runs the call the search waits for
                 const long long tw0 = clock64();
                 __nanosleep(100);
-                if (lane == 0) atomicAdd(&A.ctl->dbg[4], (unsigned long long)(clock64() - tw0));
+                if (lane == 0) atomicAdd(&A.ctl->diag[DIAG_OWNER_WAIT_CYCLES], (unsigned long long)(clock64() - tw0));
                 continue;
             }
             // RQ_FINDWORK: the call the search waits for runs on a helper; take the next unclaimed call of this pair instead
@@ -744,7 +744,7 @@ __device__ __forceinline__ void schedule(Cta& c) {
             int s = -1;
             const int o = find_help(c, &s);
             if (o >= 0) {
-                if (lane == 0) { os.action = ACT_CALL; os.actOwner = o; os.actSlot = s; os.actCancel = 1; atomicAdd(&A.ctl->dbg[2], (unsigned long long)(clock64() - th0)); atomicAdd(&A.ctl->dbg[5], 1ull);
+                if (lane == 0) { os.action = ACT_CALL; os.actOwner = o; os.actSlot = s; os.actCancel = 1; atomicAdd(&A.ctl->diag[DIAG_HELP_SCAN_CYCLES], (unsigned long long)(clock64() - th0)); atomicAdd(&A.ctl->diag[DIAG_HELPER_CALLS], 1ull);
                                  unsigned long long now; asm volatile("mov.u64 %0, %%globaltimer;" : "=l"(now)); atomicAdd(&A.ctl->helpHist[min(255ull, (now - A.ctl->t0ns) / 4000000ull)], 1); }
                 __syncwarp();
                 return;
@@ -758,7 +758,7 @@ __device__ __forceinline__ void schedule(Cta& c) {
             if (done) { if (lane == 0) os.action = ACT_EXIT; __syncwarp(); return; }
         }
         __nanosleep(os.pair >= 0 ? 200 : 500);
-        if (lane == 0) atomicAdd(&A.ctl->dbg[os.pair >= 0 ? 4 : 3], (unsigned long long)(clock64() - th0));
+        if (lane == 0) atomicAdd(&A.ctl->diag[os.pair >= 0 ? DIAG_OWNER_WAIT_CYCLES : DIAG_IDLE_CYCLES], (unsigned long long)(clock64() - th0));
         __syncwarp();
     }
 }
@@ -801,7 +801,7 @@ search_kernel(const SearchArgs A) {
             icp_fused_body(A.pairs, icp, icpTile, icpCap);
             __syncthreads();
             icp_fused_body(A.pairs, icp + 1, icpTile, icpCap);
-            if (tid == 0) { atomicAdd(reinterpret_cast<unsigned long long*>(A.genCounter) + 1 + 6, 2ull); atomicAdd(&A.ctl->dbg[7], (unsigned long long)(clock64() - ti0)); }
+            if (tid == 0) { atomicAdd(&A.ctr->icpRequests, 2ull); atomicAdd(&A.ctl->diag[DIAG_ICP_CYCLES], (unsigned long long)(clock64() - ti0)); }
             continue;
         }
         // ACT_CALL: one request out of slot (actOwner, actSlot)
@@ -810,17 +810,17 @@ search_kernel(const SearchArgs A) {
             if (tid < (int)(sizeof(InnerProb) / 4)) reinterpret_cast<unsigned*>(&s_pr)[tid] = reinterpret_cast<const volatile unsigned*>(&sl->pr)[tid];
             if (tid == 32) { s_cancel.word = os.actCancel ? &A.hdrs[os.actOwner].gen : nullptr; s_cancel.gen = os.actCancel ? ld_vol(&sl->gen) : 0u; s_cancel.flag = 0; }
         }
-        inner_call<EXACT, SMEM, GS, CT, true>(A.pairs, s_pr, s_out, s_gbar, cx, s_cancel, A.heaps, A.heapCap, A.gscratch, A.gstride, A.NdP, A.NdQ, A.useSmem, A.memo, A.memoCap, A.genCounter, A.gridOff, A.S3p);
+        inner_call<EXACT, SMEM, GS, CT, true>(A.pairs, s_pr, s_out, s_gbar, cx, s_cancel, A.heaps, A.heapCap, A.gscratch, A.gstride, A.NdP, A.NdQ, A.useSmem, A.memo, A.memoCap, A.ctr, A.gridOff, A.S3p);
         if (warp == 0) {
             SearchSlot* sl = A.slots + (size_t)os.actOwner * SR_NSLOT + os.actSlot;
             __syncwarp();
             if (lane < 16) reinterpret_cast<volatile unsigned*>(&sl->out)[lane] = reinterpret_cast<const unsigned*>(&s_out)[lane];
             __threadfence();
             __syncwarp();
-            if (lane == 0) { st_vol(A.states + (size_t)os.actOwner * SR_NSLOT + os.actSlot, SL_DONE); if (os.actCancel && s_out.status == 7) atomicAdd(&A.ctl->dbg[6], 1ull); }
+            if (lane == 0) { st_vol(A.states + (size_t)os.actOwner * SR_NSLOT + os.actSlot, SL_DONE); if (os.actCancel && s_out.status == 7) atomicAdd(&A.ctl->diag[DIAG_HELPER_ABANDONED], 1ull); }
         }
     }
-    if (tid == 0) { unsigned long long* dstat = reinterpret_cast<unsigned long long*>(A.genCounter) + 1; atomicAdd(dstat + 4, (unsigned long long)s_tIdle); atomicAdd(dstat + 7, (unsigned long long)(clock64() - s_tStart)); }
+    if (tid == 0) { atomicAdd(&A.ctr->idleCycles, (unsigned long long)s_tIdle); atomicAdd(&A.ctr->ctaCycles, (unsigned long long)(clock64() - s_tStart)); }
 }
 
 typedef void (*search_kernel_t)(const SearchArgs);

@@ -11,7 +11,7 @@ size_t goicp_bnb_smem_floats(int NdP, int NdQ, bool exact, bool needMd, bool nee
 int goicp_inner_bnb_occupancy(size_t smemBytes, int exact, int threads, int useSmem, int ct);
 cudaError_t goicp_launch_inner_bnb(const PairDev* pairs, const InnerProb* probs, InnerOut* outs, int nprob, int* counter,
                                    HeapEnt* heaps, int heapCap, int maxCtas, float* gscratch, size_t gstride,
-                                   int NdP, int NdQ, size_t smemBytes, int useSmem, int gridOff, int S3p, int exact, int ct, int threads, void* memo, int memoCap, unsigned* genCounter, cudaStream_t st, int* ctasLaunched);
+                                   int NdP, int NdQ, size_t smemBytes, int useSmem, int gridOff, int S3p, int exact, int ct, int threads, void* memo, int memoCap, DevCounters* ctr, cudaStream_t st, int* ctasLaunched);
 cudaError_t goicp_launch_eval_bounds(const PairDev* pairs, int pair, const float* Rs, const int* levels, const WaveCube* cubes,
                                      int nt, float* ub, float* lb, int* incomp_mm, int* fpfh_mm, float* scratch, int nwarps,
                                      cudaStream_t st);

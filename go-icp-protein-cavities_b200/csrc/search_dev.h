@@ -26,11 +26,18 @@ struct alignas(128) OwnerHdr {
     unsigned nQueued;    // slots in state queued (a hint for helpers; may be transiently off by the calls being claimed)
     unsigned pad;
 };
+// SearchCtl::diag: CTA cycles and event counts, by index rather than field name because the kernel picks some of them at run time
+enum SearchDiag {
+    DIAG_OWNER_CYCLES, DIAG_PUBLISH_CYCLES, DIAG_HELP_SCAN_CYCLES, DIAG_IDLE_CYCLES, DIAG_OWNER_WAIT_CYCLES,   // CTA cycles: OuterBnB state machine, publishing speculative calls, looking for calls to help with, idle (no pair), owner waiting for a helper's result
+    DIAG_HELPER_CALLS, DIAG_HELPER_ABANDONED, DIAG_ICP_CYCLES,   // calls run for another owner, of which abandoned; CTA cycles in ICP
+    DIAG_PAIRS_OUT_LAST_NS, DIAG_PAIRS_OUT_FIRST_NS,   // ns after the start when the last / the first CTA found the pair counter run out
+    DIAG_PRUNE_CYCLES, DIAG_POP_CYCLES,   // CTA cycles: queue pruning after improvements, rotation-queue pops
+    DIAG_POPS_AHEAD, DIAG_POPS_NOT_AHEAD, DIAG_CHILD_READY, DIAG_CHILD_WAITED,   // rotation nodes popped with / without calls made ahead; children whose result was there when the search reached them / waited for
+    DIAG_N
+};
 struct SearchCtl {
     int nextPair, pairsDone, owners, pad;
-    // diagnostics (GOICP_DEBUG): CTA cycles by activity and 4 ms histograms over the kernel's run time
-    unsigned long long dbg[16];      // [0] OuterBnB state machine [1] publishing speculative calls [2] looking for calls to help with [3] idle, no pair
-                                     // [4] owner waiting for a helper's result [5] calls run for another owner [6] of which abandoned [7] ICP [8] ns when the pair counter ran out
+    unsigned long long diag[DIAG_N];   // diagnostics (GOICP_DEBUG), indexed by SearchDiag
     unsigned long long t0ns;
     int finishHist[256], helpHist[256];
     unsigned wantHelp[32];           // bit per CTA: it has published calls nobody has claimed yet (a hint)
@@ -59,7 +66,7 @@ struct SearchArgs {
     int deepCalls;       // a pair asks for help while unclaimed pairs remain once it has consumed this many InnerBnB calls (one more group per multiple)
     SearchCtl* ctl; OwnerHdr* hdrs; SearchSlot* slots; unsigned* states; void* rq; int rqCap; IcpState* icp; PairOut* outs;
     // inner_call
-    HeapEnt* heaps; int heapCap; float* gscratch; size_t gstride; int NdP, NdQ, useSmem; uint4* memo; int memoCap; unsigned* genCounter; int gridOff, S3p;
+    HeapEnt* heaps; int heapCap; float* gscratch; size_t gstride; int NdP, NdQ, useSmem; uint4* memo; int memoCap; DevCounters* ctr; int gridOff, S3p;
 };
 
 size_t goicp_search_slot_bytes();

@@ -11,4 +11,4 @@ reg = g.GoICP(z["model_xyz"], z["data_xyz"], g.shipped_config(), **clouds)
 reg.BuildDT(); reg.set_nd(int(z["nd"])); reg.Initialize()
 o = po.Oracle("port", z["model_xyz"], z["data_xyz"], po.shipped_config(), **clouds); o.build_dt(); o.set_nd(int(z["nd"])); o.initialize()
 e, R, t, corr = reg.ICP(np.eye(3), np.zeros(3)); eo, Ro, to, co = o.icp(np.eye(3), np.zeros(3))
-print("fused env", os.environ.get("GOICP_ICP_FUSED"), "err", e, eo, "dR", np.abs(R - Ro).max(), "corr eq", (corr == co).mean())
+print("err", e, eo, "dR", np.abs(R - Ro).max(), "corr eq", (corr == co).mean())
