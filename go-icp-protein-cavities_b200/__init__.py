@@ -65,7 +65,8 @@ ABI_SYMBOLS = [
     "goicp_set_model", "goicp_set_data", "goicp_set_params", "goicp_build_dt", "goicp_build_dt_replay", "goicp_dt_upload",
     "goicp_dt_download", "goicp_dt_distance", "goicp_set_nd", "goicp_initialize", "goicp_get_weights", "goicp_get_maxrotdis",
     "goicp_get_thresholds", "goicp_eval_bounds", "goicp_eval_inclusion", "goicp_inner_bnb", "goicp_icp", "goicp_register", "goicp_outer_bnb", "goicp_last_trace",
-    "goicp_set_options", "goicp_set_search_mode", "goicp_register_batch", "goicp_batch_upload", "goicp_batch_run", "goicp_get_timings",
+    "goicp_set_options", "goicp_set_search_mode", "goicp_register_batch", "goicp_batch_upload", "goicp_batch_upload_dev", "goicp_batch_run",
+    "goicp_get_cells", "goicp_get_timings",
     "goicp_set_batch_options", "goicp_get_stats", "goicp_set_frontier_sharding", "goicp_test_exchange",
     "goicp_normalize_cloud", "goicp_scale_cloud", "goicp_rescale_translation", "goicp_apply_rigid", "goicp_rmsd",
 ]
@@ -116,7 +117,10 @@ def lib():
     L.goicp_set_search_mode.argtypes = [vp, C.c_int32, C.c_int32]
     L.goicp_register_batch.argtypes = [vp, C.POINTER(Params), C.c_int32, C.POINTER(PairDesc), C.POINTER(Result)]
     L.goicp_batch_upload.argtypes = [vp, C.POINTER(Params), C.c_int32, C.POINTER(PairDesc)]
+    L.goicp_batch_upload_dev.argtypes = [vp, C.POINTER(Params), C.c_int32, C.POINTER(PairDesc)]
     L.goicp_batch_run.argtypes = [vp, C.POINTER(Result)]
+    u8p = C.POINTER(C.c_uint8)
+    L.goicp_get_cells.argtypes = [vp, C.c_int32, ip, ip, ip, C.POINTER(C.c_uint32), u8p, u8p, C.POINTER(DTInfo)]
     L.goicp_get_timings.argtypes = [vp, fp, C.POINTER(C.c_int64)]
     L.goicp_set_batch_options.argtypes = [vp, C.c_int32, C.c_int32]
     L.goicp_get_stats.argtypes = [vp, dp]
@@ -280,6 +284,58 @@ class Engine:
         self.check(self.L.goicp_register_batch(self.h, C.byref(params), len(pairs), arr, res))
         return [_result_dict(r) for r in res]
 
+    def batch_upload_tensors(self, params, model_xyz, model_offsets, data_xyz, data_offsets, model_c=None, data_c=None,
+                             model_fpfh=None, data_fpfh=None, nd=None):
+        """goicp_batch_upload_dev from packed ragged CUDA tensors: pair k's model is model_xyz[model_offsets[k]:model_offsets[k+1]]
+        (float32 [sum Nm, 3]), likewise the data cloud; colours int32 [sum N], c-FPFH rows float32 [sum N, 41]; offsets are CPU
+        int64 [P+1] (the sizes are needed on the host); nd: per-pair NdDownsampled (0 = all) or None.  The clouds are read
+        after the work already queued on torch's current stream of their device; batch_run() follows."""
+        import torch
+        dev = _cuda_tensor(torch, model_xyz, "model_xyz", torch.float32, (None, 3)).device
+        _cuda_tensor(torch, data_xyz, "data_xyz", torch.float32, (None, 3), dev)
+        mo = _offsets(torch, model_offsets, model_xyz.shape[0], "model_offsets")
+        do = _offsets(torch, data_offsets, data_xyz.shape[0], "data_offsets")
+        if len(mo) != len(do):
+            raise ValueError("model_offsets and data_offsets describe different numbers of pairs")
+        npairs = len(mo) - 1
+        tm = dict(model_c=(model_c, torch.int32, (int(mo[-1]),)), model_fpfh=(model_fpfh, torch.float32, (int(mo[-1]), 41)),
+                  data_c=(data_c, torch.int32, (int(do[-1]),)), data_fpfh=(data_fpfh, torch.float32, (int(do[-1]), 41)))
+        for name, (t, dt, shape) in tm.items():
+            if t is not None:
+                _cuda_tensor(torch, t, name, dt, shape, dev)
+        if nd is not None and len(nd) != npairs:
+            raise ValueError(f"nd has {len(nd)} entries for {npairs} pairs")
+        arr = (PairDesc * npairs)()
+
+        def at(t, off, row):
+            return None if t is None else C.cast(C.c_void_p(t.data_ptr() + int(off) * row), C.POINTER(C.c_float if t.dtype == torch.float32 else C.c_int32))
+        for k in range(npairs):
+            arr[k] = PairDesc(at(model_xyz, mo[k], 12), at(model_c, mo[k], 4), at(model_fpfh, mo[k], 164), int(mo[k + 1] - mo[k]),
+                              at(data_xyz, do[k], 12), at(data_c, do[k], 4), at(data_fpfh, do[k], 164), int(do[k + 1] - do[k]),
+                              0 if nd is None else int(nd[k]))
+        torch.cuda.current_stream(dev).synchronize()   # the clouds may still be written on torch's stream
+        self._npairs = npairs
+        self.check(self.L.goicp_batch_upload_dev(self.h, C.byref(params), npairs, arr))
+
+    def register_batch_tensors(self, params, *args, **kw):
+        """batch_upload_tensors + batch_run: the per-pair result dicts of register_batch"""
+        self.batch_upload_tensors(params, *args, **kw)
+        return self.batch_run()
+
+    def get_cells(self, pair, nm, ndall):
+        """goicp_get_cells: the cell lists, colour masks and colour indices the grid of `pair` (nm model and ndall data points)
+        was built from"""
+        info = DTInfo()
+        self.check(self.L.goicp_get_cells(self.h, pair, None, None, None, None, None, None, C.byref(info)))
+        nc = info.ncells
+        start = np.zeros(nc + 1, np.int32)
+        self.check(self.L.goicp_get_cells(self.h, pair, None, _p(start, C.c_int32), None, None, None, None, None))
+        vox, pts, cmask = np.zeros(nc, np.int32), np.zeros(int(start[-1]), np.int32), np.zeros(nc + 1, np.uint32)
+        mprop, dprop = np.zeros(nm, np.uint8), np.zeros(ndall, np.uint8)
+        self.check(self.L.goicp_get_cells(self.h, pair, _p(vox, C.c_int32), None, _p(pts, C.c_int32), _p(cmask, C.c_uint32),
+                                          _p(mprop, C.c_uint8), _p(dprop, C.c_uint8), None))
+        return dict(cell_vox=vox, cell_start=start, cell_pts=pts, cmask=cmask, mprop=mprop, dprop=dprop, info=info)
+
     # ---- Transformation (transformation.cpp) ----
     def normalizeMolCloud(self, xyz):
         """:311 -- returns (centred cloud, mean, max norm)"""
@@ -311,6 +367,33 @@ class Engine:
         out = C.c_float()
         self.check(self.L.goicp_rmsd(self.h, _p(a, C.c_double), _p(b, C.c_double), len(a), C.byref(out)))
         return float(out.value)
+
+
+def _cuda_tensor(torch, t, name, dtype, shape, device=None):
+    """t must be a contiguous CUDA tensor of `dtype` with `shape` (None: any length), on `device` when given"""
+    if not torch.is_tensor(t) or not t.is_cuda:
+        raise ValueError(f"{name} must be a CUDA tensor")
+    if t.dtype != dtype:
+        raise ValueError(f"{name} must be {dtype}, not {t.dtype}")
+    if not t.is_contiguous():
+        raise ValueError(f"{name} must be contiguous")
+    if t.dim() != len(shape) or any(w is not None and w != v for w, v in zip(shape, t.shape)):
+        raise ValueError(f"{name} has shape {tuple(t.shape)}, expected {tuple('N' if w is None else w for w in shape)}")
+    if device is not None and t.device != device:
+        raise ValueError(f"{name} is on {t.device}, the clouds on {device}")
+    return t
+
+
+def _offsets(torch, o, n, name):
+    """CPU int64 [P+1] offsets into an array of n rows: 0 first, n last, every pair non-empty"""
+    if not torch.is_tensor(o) or o.is_cuda or o.dtype != torch.int64 or o.dim() != 1 or len(o) < 2:
+        raise ValueError(f"{name} must be a CPU int64 tensor of P+1 offsets")
+    a = o.numpy()
+    if a[0] != 0 or a[-1] != n or (np.diff(a) < 1).any():
+        raise ValueError(f"{name} must rise strictly from 0 to {n}")
+    if np.diff(a).max() >= 2 ** 31:
+        raise ValueError(f"{name}: a cloud has 2^31 points or more")
+    return a
 
 
 def _result_dict(r):

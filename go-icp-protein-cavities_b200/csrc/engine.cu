@@ -4,6 +4,7 @@
 // otherwise by one of the host wave schedulers of engine_search.cu.  DESIGN.md section 5 says which runs when.
 //
 // There is no CPU fallback anywhere in this file: every numeric result comes from a kernel.
+#include <cuda.h>   // types of the driver range query (no link dependency)
 #include "engine_internal.h"
 
 std::string g_create_error;
@@ -13,6 +14,34 @@ static goicp_status ensure_single(Eng* h) {
     if (h->probs.size() != 1) return fail(h, GOICP_ERR_ARG, "no single registration problem set (call goicp_set_model/goicp_set_data)");
     return GOICP_OK;
 }
+
+// Validation of caller buffers in device memory.  cudaPointerGetAttributes says whether a pointer is device or managed
+// memory of which device; the driver's range query (reached through the runtime, so the library does not link libcuda)
+// gives the whole allocation, so that the buffers of a packed batch cost one query per allocation, not one per pair.
+struct DevRanges {
+    std::vector<std::pair<uintptr_t, uintptr_t>> ok;   // validated allocations [begin, end)
+    // NULL if [ptr, ptr + bytes) lies in one device or managed allocation of `device`, else the reason
+    const char* check(int device, const void* ptr, size_t bytes) {
+        const uintptr_t b = (uintptr_t)ptr, e = b + bytes;
+        for (auto& r : ok) if (b >= r.first && e <= r.second) return nullptr;
+        cudaPointerAttributes a;
+        if (cudaPointerGetAttributes(&a, ptr) != cudaSuccess) { cudaGetLastError(); return "is not memory"; }
+        if ((a.type != cudaMemoryTypeDevice && a.type != cudaMemoryTypeManaged) || a.device != device) return "is not device or managed memory";
+        typedef CUresult (*RangeFn)(CUdeviceptr*, size_t*, CUdeviceptr);
+        static RangeFn range = nullptr;
+        if (!range) {
+            void* fn = nullptr; cudaDriverEntryPointQueryResult q;
+            if (cudaGetDriverEntryPoint("cuMemGetAddressRange", &fn, cudaEnableDefault, &q) != cudaSuccess || q != cudaDriverEntryPointSuccess || !fn) return "cannot be checked (no driver range query)";
+            range = (RangeFn)fn;
+        }
+        CUdeviceptr base = 0; size_t size = 0;
+        if (a.type == cudaMemoryTypeManaged) { base = (CUdeviceptr)b; size = bytes; }   // managed: no range query; this buffer only
+        else if (range(&base, &size, (CUdeviceptr)b) != CUDA_SUCCESS) return "is not in a device allocation";
+        if (b < base || e > base + size) return "extends past its allocation";
+        ok.emplace_back((uintptr_t)base, (uintptr_t)(base + size));
+        return nullptr;
+    }
+};
 }  // namespace
 
 // =====================================================================================================================
@@ -46,7 +75,8 @@ goicp_status goicp_create(goicp_handle* out, int device, void* stream_or_null) {
     h->device = device; h->numSM = prop.multiProcessorCount;
     if (stream_or_null) { h->stream = (cudaStream_t)stream_or_null; h->ownStream = false; }
     else { if ((e = cudaStreamCreateWithFlags(&h->stream, cudaStreamNonBlocking)) != cudaSuccess) { delete h; return fail(nullptr, GOICP_ERR_CUDA, "cudaStreamCreate: %s", cudaGetErrorString(e)); } h->ownStream = true; }
-    if ((e = goicp_preload_bnb()) != cudaSuccess || (e = goicp_preload_dt()) != cudaSuccess || (e = goicp_preload_icp()) != cudaSuccess || (e = goicp_preload_misc()) != cudaSuccess || (e = goicp_preload_search()) != cudaSuccess) {
+    if ((e = goicp_preload_bnb()) != cudaSuccess || (e = goicp_preload_dt()) != cudaSuccess || (e = goicp_preload_icp()) != cudaSuccess || (e = goicp_preload_misc()) != cudaSuccess || (e = goicp_preload_search()) != cudaSuccess ||
+        (e = goicp_preload_prep()) != cudaSuccess) {
         delete h; return fail(nullptr, GOICP_ERR_CUDA, "kernel preload failed: %s (library built for sm_100a only)", cudaGetErrorString(e));
     }
     if (h->devCounters.ensure(sizeof(DevCounters)) != cudaSuccess || cudaMemset(h->devCounters.p, 0, sizeof(DevCounters)) != cudaSuccess) { delete h; return fail(nullptr, GOICP_ERR_CUDA, "device allocation failed"); }
@@ -60,9 +90,9 @@ void goicp_destroy(goicp_handle h) {
     if (!h) return;
     cudaSetDevice(h->device);
     cudaStreamSynchronize(h->stream);
-    DevBuf* bufs[] = {&h->arenaIn, &h->arenaWork, &h->dPairs, &h->dTmp, &h->dTmp2, &h->dTmp3, &h->dSepBits, &h->dSepNx, &h->dSepNxy, &h->dSepCid, &h->sCtl, &h->sHdrs, &h->sSlots, &h->sStates, &h->sRq, &h->sIcp, &h->sOuts};
+    DevBuf* bufs[] = {&h->arenaIn, &h->arenaWork, &h->dPairs, &h->dTmp, &h->dTmp2, &h->dTmp3, &h->dSepBits, &h->dSepNx, &h->dSepNxy, &h->dSepCid, &h->dRaw, &h->dPrep, &h->sCtl, &h->sHdrs, &h->sSlots, &h->sStates, &h->sRq, &h->sIcp, &h->sOuts};
     for (DevBuf* b : bufs) b->release();
-    h->hStage.release(); h->hPairs.release(); h->hOuts.release(); h->qHeaps.release(); h->qScratch.release(); h->qMemo.release(); h->devCounters.release();
+    h->hStage.release(); h->hPairs.release(); h->hPrep.release(); h->hOuts.release(); h->qHeaps.release(); h->qScratch.release(); h->qMemo.release(); h->devCounters.release();
     h->main.release();
     for (auto& w : h->workers) w->release();
     if (h->ownStream) cudaStreamDestroy(h->stream);
@@ -74,7 +104,7 @@ goicp_status goicp_set_model(goicp_handle h, const float* xyz, const int32_t* c,
     if (h->probs.size() != 1) { h->probs.clear(); h->probs.resize(1); }
     Problem& P = h->probs[0];
     set_cloud(P.mxyz, P.mc, P.mf, xyz, c, fpfh41, Nm); P.Nm = Nm;
-    P.prepared = P.dt_built = P.initialized = false;
+    P.uploaded = P.prepared = P.dt_built = P.initialized = false;
     return GOICP_OK;
 }
 goicp_status goicp_set_data(goicp_handle h, const float* xyz, const int32_t* c, const float* fpfh41, int32_t Nd) {
@@ -82,7 +112,7 @@ goicp_status goicp_set_data(goicp_handle h, const float* xyz, const int32_t* c, 
     if (h->probs.size() != 1) { h->probs.clear(); h->probs.resize(1); }
     Problem& P = h->probs[0];
     set_cloud(P.dxyz, P.dc, P.df, xyz, c, fpfh41, Nd); P.NdAll = Nd; P.Nd = Nd;
-    P.prepared = P.dt_built = P.initialized = false;
+    P.uploaded = P.prepared = P.dt_built = P.initialized = false;
     return GOICP_OK;
 }
 goicp_status goicp_set_params(goicp_handle h, const goicp_params* p) {
@@ -90,7 +120,7 @@ goicp_status goicp_set_params(goicp_handle h, const goicp_params* p) {
     const bool gridChanged = !h->haveParams || p->distTransSize != h->params.distTransSize || p->distTransExpandFactor != h->params.distTransExpandFactor ||
                              (p->trimFraction < 0.001) != (h->params.trimFraction < 0.001) ||
                              p->cfpfh != h->params.cfpfh || p->regularizationFPFH != h->params.regularizationFPFH ||
-                             (p->regularizationNeighbors > 0) != (h->params.regularizationNeighbors > 0);   // every key the arena layout (upload_problems) depends on
+                             (p->regularizationNeighbors > 0) != (h->params.regularizationNeighbors > 0);   // every key K1 or the arena layout depends on
     h->params = *p; h->haveParams = true;
     for (auto& P : h->probs) { P.initialized = false; if (gridChanged) P.prepared = P.dt_built = false; }
     return GOICP_OK;
@@ -148,13 +178,19 @@ goicp_status goicp_dt_download(goicp_handle h, float* dist, int32_t* nearest, in
     cudaSetDevice(h->device);
     const int S = P.info.size; const size_t S3 = (size_t)S * S * S;
     if (dist) CU(cudaMemcpyAsync(dist, P.dev.g.dist, sizeof(float) * S3, cudaMemcpyDeviceToHost, h->stream));
-    std::vector<int> vn;
+    std::vector<int> vn, cv, cc;
     if (nearest) { vn.resize(S3); CU(cudaMemcpyAsync(vn.data(), P.dev.g.vnear, sizeof(int) * S3, cudaMemcpyDeviceToHost, h->stream)); }
+    const int nc = P.info.ncells;
+    if (cellc && nc > 0) {
+        cv.resize(nc); cc.resize(nc);
+        CU(cudaMemcpyAsync(cv.data(), P.dev.g.cell_vox, sizeof(int) * nc, cudaMemcpyDeviceToHost, h->stream));
+        CU(cudaMemcpyAsync(cc.data(), P.cell_col, sizeof(int) * nc, cudaMemcpyDeviceToHost, h->stream));
+    }
     CU(cudaStreamSynchronize(h->stream));
     if (nearest) for (size_t i = 0; i < S3; i++) { int v = vn[i]; nearest[3 * i] = v % S; nearest[3 * i + 1] = (v / S) % S; nearest[3 * i + 2] = v / (S * S); }
     if (cellc) {
         for (size_t i = 0; i < S3; i++) cellc[i] = -2;
-        for (int c = 0; c < P.info.ncells; c++) cellc[P.cell_vox[c]] = P.cell_colour[c];
+        for (int c = 0; c < nc; c++) cellc[cv[c]] = cc[c];
     }
     return GOICP_OK;
 }
@@ -321,30 +357,73 @@ goicp_status goicp_outer_bnb(goicp_handle h, goicp_result* out) {
 const char* goicp_last_trace(goicp_handle h) { return h ? h->trace.c_str() : ""; }
 
 // ---- batch -----------------------------------------------------------------------------------------------------------
-goicp_status goicp_batch_upload(goicp_handle h, const goicp_params* p, int32_t npairs, const goicp_pair_desc* pairs) {
+static goicp_status batch_upload_impl(goicp_handle h, const goicp_params* p, int32_t npairs, const goicp_pair_desc* pairs, bool onDevice) {
     if (!h || !p || npairs < 1 || !pairs) return GOICP_ERR_ARG;
     cudaSetDevice(h->device);
-    h->params = *p; h->haveParams = true;
-    h->probs.clear(); h->probs.resize(npairs);
     for (int i = 0; i < npairs; i++) {
         const goicp_pair_desc& d = pairs[i];
         if (!d.model_xyz || !d.data_xyz || d.Nm < 1 || d.NdAll < 1) return fail(h, GOICP_ERR_ARG, "pair %d: empty cloud", i);
     }
-    const bool wantF = p->cfpfh != 0;   // descriptors are only copied when the configuration uses them
-    parallel_for(npairs, [&](int i) {
+    if (onDevice) {   // every buffer must lie inside one allocation of device or managed memory of this handle's device
+        const bool wantF = p->cfpfh != 0;
+        DevRanges ok;
+        for (int i = 0; i < npairs; i++) {
+            const goicp_pair_desc& d = pairs[i];
+            const size_t m = d.Nm, n = d.NdAll, F = sizeof(float) * GOICP_NBINS;
+            const struct { const void* ptr; size_t bytes; const char* name; } bufs[6] = {
+                {d.model_xyz, 12 * m, "model_xyz"}, {d.model_c, 4 * m, "model_c"}, {wantF ? d.model_fpfh : nullptr, F * m, "model_fpfh"},
+                {d.data_xyz, 12 * n, "data_xyz"}, {d.data_c, 4 * n, "data_c"}, {wantF ? d.data_fpfh : nullptr, F * n, "data_fpfh"}};
+            for (const auto& b : bufs) {
+                if (!b.ptr) continue;
+                const char* why = ok.check(h->device, b.ptr, b.bytes);
+                if (why) return fail(h, GOICP_ERR_ARG, "pair %d: %s %s of device %d", i, b.name, why, h->device);
+            }
+        }
+    }
+    h->params = *p; h->haveParams = true;
+    h->probs.clear(); h->probs.resize(npairs);
+    for (int i = 0; i < npairs; i++) {
         const goicp_pair_desc& d = pairs[i]; Problem& P = h->probs[i];
-        set_cloud(P.mxyz, P.mc, P.mf, d.model_xyz, d.model_c, wantF ? d.model_fpfh : nullptr, d.Nm); P.Nm = d.Nm;
-        set_cloud(P.dxyz, P.dc, P.df, d.data_xyz, d.data_c, wantF ? d.data_fpfh : nullptr, d.NdAll); P.NdAll = d.NdAll;
-        P.Nd = (d.Nd > 0 && d.Nd <= d.NdAll) ? d.Nd : d.NdAll;
-    });
+        P.Nm = d.Nm; P.NdAll = d.NdAll; P.Nd = (d.Nd > 0 && d.Nd <= d.NdAll) ? d.Nd : d.NdAll;
+    }
     goicp_status s;
+    if ((s = upload_clouds(h, pairs, onDevice))) return s;
     if ((s = prepare_all(h))) return s;
     CU(cudaStreamSynchronize(h->stream));
     return GOICP_OK;
 }
+goicp_status goicp_batch_upload(goicp_handle h, const goicp_params* p, int32_t npairs, const goicp_pair_desc* pairs) {
+    return batch_upload_impl(h, p, npairs, pairs, false);
+}
+goicp_status goicp_batch_upload_dev(goicp_handle h, const goicp_params* p, int32_t npairs, const goicp_pair_desc* pairs) {
+    return batch_upload_impl(h, p, npairs, pairs, true);
+}
+goicp_status goicp_get_cells(goicp_handle h, int32_t pair, int32_t* cell_vox, int32_t* cell_start, int32_t* cell_pts, uint32_t* cmask,
+                             uint8_t* mprop, uint8_t* dprop, goicp_dt_info* info) {
+    if (!h) return GOICP_ERR_ARG;
+    if (pair < 0 || pair >= (int)h->probs.size()) return fail(h, GOICP_ERR_ARG, "get_cells: pair %d out of range", pair);
+    Problem& P = h->probs[pair];
+    if (!P.prepared) return fail(h, GOICP_ERR_ARG, "get_cells before the grid is prepared (batch upload or build_dt)");
+    cudaSetDevice(h->device);
+    const int nc = P.info.ncells;
+    std::vector<int> start(nc + 1);
+    CU(cudaMemcpyAsync(start.data(), P.dev.cell_start, sizeof(int) * (nc + 1), cudaMemcpyDeviceToHost, h->stream));
+    if (cell_vox && nc) CU(cudaMemcpyAsync(cell_vox, P.dev.g.cell_vox, sizeof(int) * nc, cudaMemcpyDeviceToHost, h->stream));
+    if (cmask) CU(cudaMemcpyAsync(cmask, P.dev.g.cmask, sizeof(uint32_t) * (nc + 1), cudaMemcpyDeviceToHost, h->stream));
+    if (mprop) CU(cudaMemcpyAsync(mprop, P.dev.mprop, P.Nm, cudaMemcpyDeviceToHost, h->stream));
+    if (dprop) CU(cudaMemcpyAsync(dprop, P.dev.dprop, P.NdAll, cudaMemcpyDeviceToHost, h->stream));
+    CU(cudaStreamSynchronize(h->stream));
+    if (cell_start) memcpy(cell_start, start.data(), sizeof(int) * (nc + 1));
+    if (cell_pts && start[nc] > 0) {
+        CU(cudaMemcpyAsync(cell_pts, P.dev.cell_pts, sizeof(int) * start[nc], cudaMemcpyDeviceToHost, h->stream));
+        CU(cudaStreamSynchronize(h->stream));
+    }
+    if (info) *info = P.info;
+    return GOICP_OK;
+}
 goicp_status goicp_batch_run(goicp_handle h, goicp_result* results) {
     if (!h || !results) return GOICP_ERR_ARG;
-    if (h->probs.empty()) return fail(h, GOICP_ERR_ARG, "batch_run before batch_upload");
+    if (h->probs.empty() || !h->probs[0].prepared) return fail(h, GOICP_ERR_ARG, "batch_run before a successful batch_upload");
     cudaSetDevice(h->device);
     h->main.reset_timing();
     goicp_status s;

@@ -35,7 +35,36 @@ cudaError_t goicp_launch_scale(double* xyz, int n, double scale, cudaStream_t st
 cudaError_t goicp_launch_apply_rigid(const double* xyz, int n, const double* Rt, double* out, cudaStream_t st);
 cudaError_t goicp_launch_rescale(const double* in19, double* out3, cudaStream_t st);
 cudaError_t goicp_launch_rmsd(const double* a, const double* b, int n, double* terms, float* out, cudaStream_t st);
+// k_prep.cu: K1 (packing of the raw clouds, bounding cube, colour dictionary, seeding, cell lists, colour masks)
+enum { PREP_OK = 0, PREP_DEGENERATE = 1, PREP_COLOURS = 2 };
+struct PrepSummary {          // what the host reads back after K1, per pair
+    int status;               // PREP_*
+    int ncells, ncolours, pad;
+    double xMin, xMax, yMin, yMax, zMin, zMax, scale;
+};
+struct PrepPair {
+    const float *rmxyz, *rdxyz;          // raw clouds: AoS xyz, colour codes or NULL, c-FPFH rows or NULL (read by the pack only)
+    const int *rmc, *rdc;
+    const float *rmf, *rdf;
+    int Nm, NdAll;
+    float *mx, *my, *mz, *dx, *dy, *dz;  // input arena: SoA clouds
+    int *mcol, *dcol;                    // colour codes (0 where none were given)
+    float *mfpfh, *dfpfh;                // descriptor rows, NULL when not kept
+    uint8_t *mprop, *dprop, *dknown;     // K1 outputs (PairDev fields of the same names)
+    int *cell_vox, *cell_start, *cell_pts, *cell_col;
+    uint32_t* cmask;
+    int *vcount, *vcid;                  // S^3 scratch (the pair's vnear / vcell of the work arena): points per voxel, then
+                                         // the scatter cursor; cell id of each occupied voxel
+    int* tmp;                            // Nm: cell members in arrival order
+};
+#define PREP_BLOCK_VOXELS 4096
+inline int goicp_prep_nblocks(int S) { return (int)(((long long)S * S * S + PREP_BLOCK_VOXELS - 1) / PREP_BLOCK_VOXELS); }
+// maxElems: the largest per-pair element count of any raw array (41 x points when descriptors are packed)
+cudaError_t goicp_launch_prep_pack(const PrepPair* pairs, int npairs, long long maxElems, cudaStream_t st);
+// bsum: npairs x goicp_prep_nblocks(S) scratch
+cudaError_t goicp_launch_prep(const PrepPair* pairs, PrepSummary* sums, long long* bsum, int npairs, int maxNm, int S, double ef, cudaStream_t st);
 // lazy-loading guards (see k_*.cu)
+cudaError_t goicp_preload_prep();
 cudaError_t goicp_preload_bnb();
 cudaError_t goicp_preload_dt();
 cudaError_t goicp_preload_icp();

@@ -173,6 +173,19 @@ goicp_status goicp_register_batch(goicp_handle h, const goicp_params* p, int32_t
  * run does DT build + Initialize + search entirely from HBM, results come back in goicp_batch_run. */
 goicp_status goicp_batch_upload(goicp_handle h, const goicp_params* p, int32_t npairs, const goicp_pair_desc* pairs);
 goicp_status goicp_batch_run(goicp_handle h, goicp_result* results);
+/* goicp_batch_upload with the six cloud pointers of every descriptor in DEVICE memory (device or managed memory of the
+ * handle's device), e.g. the storage of CUDA tensors; the descriptor array and its sizes are host memory.  The buffers are
+ * read by kernels on the handle's stream, so they are read after work already queued on that stream, and they are not read
+ * after the call returns.  A pointer that is not device or managed memory of the handle's device, or a buffer that runs
+ * past its allocation, fails with GOICP_ERR_ARG before any launch.  goicp_batch_run follows as after goicp_batch_upload. */
+goicp_status goicp_batch_upload_dev(goicp_handle h, const goicp_params* p, int32_t npairs, const goicp_pair_desc* pairs);
+/* test hook: the cell lists and colour masks of pair `pair` (0 for a single registration) once its grid is prepared
+ * (batch upload or build_dt) -- cell_vox[ncells] ascending voxel indices (z*S+y)*S+x of the occupied voxels,
+ * cell_start[ncells+1] CSR offsets into cell_pts[cell_start[ncells]] (<= Nm model point indices, ascending within a cell),
+ * cmask[ncells+1] per-cell colour masks (checkProperty, jly_goicp.cpp:1068-1092; the last entry is 0), mprop[Nm] and
+ * dprop[NdAll] the colour-dictionary index of every point, info the grid geometry.  NULL skips an output. */
+goicp_status goicp_get_cells(goicp_handle h, int32_t pair, int32_t* cell_vox, int32_t* cell_start, int32_t* cell_pts, uint32_t* cmask,
+                             uint8_t* mprop, uint8_t* dprop, goicp_dt_info* info);
 /* device-event timings (ms) and launch counts of the last batch_run / register:
  * out[0] dt build, [1] initialize, [2] inner-BnB kernels, [3] ICP kernels, [4] other; launches[0..4] likewise */
 goicp_status goicp_get_timings(goicp_handle h, float* ms5, int64_t* launches5);
