@@ -66,7 +66,7 @@ ABI_SYMBOLS = [
     "goicp_dt_download", "goicp_dt_distance", "goicp_set_nd", "goicp_initialize", "goicp_get_weights", "goicp_get_maxrotdis",
     "goicp_get_thresholds", "goicp_eval_bounds", "goicp_eval_inclusion", "goicp_inner_bnb", "goicp_icp", "goicp_register", "goicp_outer_bnb", "goicp_last_trace",
     "goicp_set_options", "goicp_set_search_mode", "goicp_register_batch", "goicp_batch_upload", "goicp_batch_upload_dev", "goicp_batch_run",
-    "goicp_get_cells", "goicp_get_timings",
+    "goicp_get_cells", "goicp_get_timings", "goicp_set_error_cutoff", "goicp_get_search_ends",
     "goicp_set_batch_options", "goicp_get_stats", "goicp_set_frontier_sharding", "goicp_test_exchange",
     "goicp_normalize_cloud", "goicp_scale_cloud", "goicp_rescale_translation", "goicp_apply_rigid", "goicp_rmsd",
 ]
@@ -122,6 +122,8 @@ def lib():
     u8p = C.POINTER(C.c_uint8)
     L.goicp_get_cells.argtypes = [vp, C.c_int32, ip, ip, ip, C.POINTER(C.c_uint32), u8p, u8p, C.POINTER(DTInfo)]
     L.goicp_get_timings.argtypes = [vp, fp, C.POINTER(C.c_int64)]
+    L.goicp_set_error_cutoff.argtypes = [vp, fp, C.c_int32]
+    L.goicp_get_search_ends.argtypes = [vp, ip, fp]
     L.goicp_set_batch_options.argtypes = [vp, C.c_int32, C.c_int32]
     L.goicp_get_stats.argtypes = [vp, dp]
     L.goicp_set_frontier_sharding.argtypes = [vp, C.c_int32, C.c_int32, ALLGATHER_FN, vp]
@@ -174,6 +176,7 @@ class Engine:
     def __init__(self, device=0, stream=None):
         self.L = lib()
         self.h = C.c_void_p()
+        self._nprobs = 0   # problems the handle holds: 1 single registration, or the pairs of the last batch upload
         st = self.L.goicp_create(C.byref(self.h), device, stream)
         if st != 0:
             raise GoICPError(st, self.L.goicp_last_error(None).decode())
@@ -243,6 +246,24 @@ class Engine:
     def set_batch_options(self, groups=-1, slots=-1):
         self.check(self.L.goicp_set_batch_options(self.h, groups, slots))
 
+    def set_error_cutoff(self, cutoffs):
+        """goicp_set_error_cutoff: end each pair's search once its error is certified above its cutoff.  `cutoffs`: a scalar for
+        every pair, an array of one value per pair of the uploaded batch (+inf: none), or None to clear.  A batch upload clears
+        them, so set them after the upload and before batch_run()."""
+        n = self._nprobs
+        if cutoffs is None:
+            self.check(self.L.goicp_set_error_cutoff(self.h, None, n))
+            return
+        a = _f32(np.broadcast_to(np.asarray(cutoffs, np.float32), (n,)) if np.ndim(cutoffs) == 0 else cutoffs)
+        self.check(self.L.goicp_set_error_cutoff(self.h, _p(a, C.c_float), len(a)))
+
+    def search_ends(self):
+        """goicp_get_search_ends: (kind int32[P], lb float32[P]) of the last batch_run / register -- kind 1 rotation queue empty,
+        2 threshold reached, 3 cutoff reached (certified above the pair's cutoff: its optimum is >= lb)"""
+        kind, lb = np.zeros(self._nprobs, np.int32), np.zeros(self._nprobs, np.float32)
+        self.check(self.L.goicp_get_search_ends(self.h, _p(kind, C.c_int32), _p(lb, C.c_float)))
+        return kind, lb
+
     # ---- batch of pairs (bo1_GoICP.py:40-54) ----
     def _descs(self, pairs):
         keep, arr = [], (PairDesc * len(pairs))()
@@ -265,12 +286,13 @@ class Engine:
     def register_batch_descs(self, params, descs):
         """goicp_register_batch on a prepared descriptor array: host buffers in, results out"""
         res = (Result * descs["n"])()
+        self._nprobs = descs["n"]
         self.check(self.L.goicp_register_batch(self.h, C.byref(params), descs["n"], descs["arr"], res))
         return res
 
     def batch_upload(self, params, pairs):
         arr, keep = self._descs(pairs)
-        self._npairs = len(pairs)
+        self._npairs = self._nprobs = len(pairs)
         self.check(self.L.goicp_batch_upload(self.h, C.byref(params), len(pairs), arr))
 
     def batch_run(self):
@@ -281,6 +303,7 @@ class Engine:
     def register_batch(self, params, pairs):
         arr, keep = self._descs(pairs)
         res = (Result * len(pairs))()
+        self._nprobs = len(pairs)
         self.check(self.L.goicp_register_batch(self.h, C.byref(params), len(pairs), arr, res))
         return [_result_dict(r) for r in res]
 
@@ -314,7 +337,7 @@ class Engine:
                               at(data_xyz, do[k], 12), at(data_c, do[k], 4), at(data_fpfh, do[k], 164), int(do[k + 1] - do[k]),
                               0 if nd is None else int(nd[k]))
         torch.cuda.current_stream(dev).synchronize()   # the clouds may still be written on torch's stream
-        self._npairs = npairs
+        self._npairs = self._nprobs = npairs
         self.check(self.L.goicp_batch_upload_dev(self.h, C.byref(params), npairs, arr))
 
     def register_batch_tensors(self, params, *args, **kw):
@@ -418,6 +441,7 @@ class GoICP:
         self.eng.check(self.L.goicp_set_params(self.h, C.byref(params)))
         self.eng.check(self.L.goicp_set_model(self.h, _p(self.pModel, C.c_float), _p(mc, C.c_int32), _p(mf, C.c_float), self.Nm))
         self.eng.check(self.L.goicp_set_data(self.h, _p(self.pData, C.c_float), _p(dc, C.c_int32), _p(df, C.c_float), self.Nd))
+        self.eng._nprobs = 1   # the handle now holds this one problem
         self.dt = None
         self.optError, self.optR, self.optT, self.optComp = None, np.eye(3), np.zeros(3), 0
 
@@ -430,6 +454,11 @@ class GoICP:
 
     def set_options(self, exact_sums=-1, spec_width=-1, use_dt_replay=-1):
         self.eng.check(self.L.goicp_set_options(self.h, exact_sums, spec_width, use_dt_replay))
+
+    def set_error_cutoff(self, tau):
+        """goicp_set_error_cutoff for this registration: Register() stops once its error is certified above tau (trace end line
+        "Cutoff reached"); None or +inf: the full search"""
+        self.eng.set_error_cutoff(tau)
 
     def BuildDT(self, replay=None):
         """GoICP::BuildDT (jly_goicp.cpp:79)"""

@@ -90,9 +90,9 @@ void goicp_destroy(goicp_handle h) {
     if (!h) return;
     cudaSetDevice(h->device);
     cudaStreamSynchronize(h->stream);
-    DevBuf* bufs[] = {&h->arenaIn, &h->arenaWork, &h->dPairs, &h->dTmp, &h->dTmp2, &h->dTmp3, &h->dSepBits, &h->dSepNx, &h->dSepNxy, &h->dSepCid, &h->dRaw, &h->dPrep, &h->sCtl, &h->sHdrs, &h->sSlots, &h->sStates, &h->sRq, &h->sIcp, &h->sOuts};
+    DevBuf* bufs[] = {&h->arenaIn, &h->arenaWork, &h->dPairs, &h->dTmp, &h->dTmp2, &h->dTmp3, &h->dSepBits, &h->dSepNx, &h->dSepNxy, &h->dSepCid, &h->dRaw, &h->dPrep, &h->sCtl, &h->sHdrs, &h->sSlots, &h->sStates, &h->sRq, &h->sIcp, &h->sOuts, &h->dCutoff};
     for (DevBuf* b : bufs) b->release();
-    h->hStage.release(); h->hPairs.release(); h->hPrep.release(); h->hOuts.release(); h->qHeaps.release(); h->qScratch.release(); h->qMemo.release(); h->devCounters.release();
+    h->hStage.release(); h->hPairs.release(); h->hPrep.release(); h->hOuts.release(); h->hCutoff.release(); h->qHeaps.release(); h->qScratch.release(); h->qMemo.release(); h->devCounters.release();
     h->main.release();
     for (auto& w : h->workers) w->release();
     if (h->ownStream) cudaStreamDestroy(h->stream);
@@ -451,6 +451,21 @@ goicp_status goicp_set_search_mode(goicp_handle h, int32_t relaxed_order, int32_
     if (!h) return GOICP_ERR_ARG;
     if (relaxed_order >= 0) h->relaxed = relaxed_order ? 1 : 0;
     if (wave_nodes >= 1) h->wave_nodes = wave_nodes;
+    return GOICP_OK;
+}
+goicp_status goicp_set_error_cutoff(goicp_handle h, const float* cutoff_or_null, int32_t n) {
+    if (!h) return GOICP_ERR_ARG;
+    if (h->probs.empty()) return fail(h, GOICP_ERR_ARG, "set_error_cutoff before any problem is set (set_model / set_data or a batch upload)");
+    if (n != (int32_t)h->probs.size()) return fail(h, GOICP_ERR_ARG, "set_error_cutoff: %d values for %d problems", n, (int)h->probs.size());
+    if (cutoff_or_null)
+        for (int i = 0; i < n; i++) if (std::isnan(cutoff_or_null[i])) return fail(h, GOICP_ERR_ARG, "set_error_cutoff: the cutoff of problem %d is NaN", i);
+    for (int i = 0; i < n; i++) h->probs[i].cutoff = cutoff_or_null ? cutoff_or_null[i] : INFINITY;
+    return GOICP_OK;
+}
+goicp_status goicp_get_search_ends(goicp_handle h, int32_t* kind, float* lb) {
+    if (!h || !kind || !lb) return GOICP_ERR_ARG;
+    if (h->probs.empty() || h->probs[0].res.endKind == 0) return fail(h, GOICP_ERR_ARG, "get_search_ends before a register or batch run");
+    for (size_t i = 0; i < h->probs.size(); i++) { kind[i] = h->probs[i].res.endKind; lb[i] = h->probs[i].res.endLb; }
     return GOICP_OK;
 }
 goicp_status goicp_set_batch_options(goicp_handle h, int32_t groups, int32_t slots) {

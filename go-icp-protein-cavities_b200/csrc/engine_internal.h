@@ -88,6 +88,7 @@ struct Problem {
     // ---- device ----
     PairDev dev{};
     size_t inBytes = 0, workBytes = 0, inOff = 0, workOff = 0;
+    float cutoff = INFINITY;             // goicp_set_error_cutoff: the search ends once the pair is certified above it
     // ---- outputs ----
     SearchResult res;
     double t_dt = 0, t_reg = 0;
@@ -168,6 +169,7 @@ struct goicp_handle_s {
     WaveCtx main;
     DevBuf qHeaps, qScratch, qMemo, devCounters;   // per-CTA slabs of the device-resident search: translation queues, staging arrays (large Nd), corner memo; DevCounters
     DevBuf sCtl, sHdrs, sSlots, sStates, sRq, sIcp, sOuts; PinBuf hOuts;   // device-resident search (k_search.cu)
+    DevBuf dCutoff; PinBuf hCutoff; bool cutoffOn = false;   // Problem::cutoff of every pair, uploaded by upload_pairdevs when one is finite
     int spec_groups = SR_NGROUP - 4;   // device-resident search: most rotation-queue nodes with speculative calls per owner CTA (0: never speculate)
     int shardRank = 0, shardN = 1; goicp_allgather_fn allgather = nullptr; void* allgatherUser = nullptr;   // frontier sharding
     std::vector<InnerOut> xSend, xRecv;

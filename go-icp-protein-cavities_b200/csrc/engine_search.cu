@@ -161,14 +161,15 @@ static void start_search(Eng* h, HostSearch& S, const IcpState& init, const IcpS
 // Advance one pair's OuterBnB as far as cached results allow; on return S.phase tells what it waits for.
 static void advance(Eng* h, HostSearch& S) {
     SearchResult& r = h->probs[S.pair].res;
-    const float SSE = h->probs[S.pair].dev.SSEThresh;
+    const float SSE = h->probs[S.pair].dev.SSEThresh, cutoff = h->probs[S.pair].cutoff;
     for (;;) {
         switch (S.phase) {
         case PH_WAIT_INIT: case PH_WAIT_ICP: case PH_DONE: return;
         case PH_POP: {
-            if (S.q.empty()) { trace_end(r.trace, true, r.optError, S.lastLb, SSE); S.phase = PH_DONE; return; }   // :670-677
+            if (S.q.empty()) { trace_end(r, END_QUEUE_EMPTY, S.lastLb, SSE, cutoff); S.phase = PH_DONE; return; }   // :670-677
             S.par = rheap_pop(S.q); r.cnt[3]++;
-            if ((r.optError - S.par.lb) <= SSE) { trace_end(r.trace, false, r.optError, S.par.lb, SSE); S.phase = PH_DONE; return; }   // :685
+            if ((r.optError - S.par.lb) <= SSE) { trace_end(r, END_THRESHOLD, S.par.lb, SSE, cutoff); S.phase = PH_DONE; return; }   // :685
+            if (S.par.lb >= cutoff) { trace_end(r, END_CUTOFF, S.par.lb, SSE, cutoff); S.phase = PH_DONE; return; }
             S.j = 0; S.phase = PH_CHILD_UB;
             break;
         }
@@ -210,7 +211,7 @@ static void advance(Eng* h, HostSearch& S) {
 // Requests of one blocked pair: the blocking call first, then speculation in the reference's expected order.
 static void gather_requests(Eng* h, HostSearch& S, int search, std::vector<InnerProb>& reqs, std::vector<ReqTag>& tags) {
     const Problem& P = h->probs[S.pair];
-    const float SSE = P.dev.SSEThresh, optError = P.res.optError;
+    const float SSE = P.dev.SSEThresh, optError = P.res.optError, cutoff = P.cutoff;
     std::unordered_set<unsigned long long> seen;
     // a call that is cached under the current incumbent or already in flight needs no request (and no rotation matrix)
     auto known = [&](const RNode& par, int j, int kind) {
@@ -253,7 +254,7 @@ static void gather_requests(Eng* h, HostSearch& S, int search, std::vector<Inner
             if (2 * pos + 1 < n && nc < 78) cand[nc++] = 2 * pos + 1;
             if (2 * pos + 2 < n && nc < 78) cand[nc++] = 2 * pos + 2;
             const RNode& nd = S.q[pos];
-            if ((optError - nd.lb) <= SSE) break;
+            if ((optError - nd.lb) <= SSE || nd.lb >= cutoff) break;   // the search ends when this node is popped
             want_children(nd, 0, false);
         }
     }
@@ -316,6 +317,8 @@ static goicp_status register_group(Eng* h, WaveCtx& c, const BnbCfg& cfg, std::a
 // optError - (smallest lower bound in the queue) <= SSEThresh (:685).  With frontier sharding (goicp_set_frontier_sharding) the
 // requests of a wave are dealt to the ranks and their results exchanged once per wave (run_inner), so every rank applies the same
 // results and holds the same queue and incumbent: the minimum over the wave's upper bounds is the per-wave "allreduce(min)".
+// An error cutoff is checked once per wave, before its pops, and only when no lower-bound call is carried over: a carried cube is
+// in no queue, so the queue's front bounds the optimum only once every cube of the domain is either queued or discarded.
 static goicp_status register_relaxed(Eng* h, WaveCtx& c, const BnbCfg& cfg, int pi) {
     Problem& P = h->probs[pi];
     SearchResult& r = P.res = SearchResult();
@@ -325,13 +328,18 @@ static goicp_status register_relaxed(Eng* h, WaveCtx& c, const BnbCfg& cfg, int 
     push_icps(icps, pi, ICP_INIT_ERROR, r);
     if ((s = run_icp(h, c, icps))) return s;
     start_search(h, S, icps[0], icps[1]);
-    const float SSE = P.dev.SSEThresh;
+    const float SSE = P.dev.SSEThresh, cutoff = P.cutoff;
     struct Item { RNode node; float R[9]; bool lbOnly; float ub; };
     std::vector<Item> items, carry;   // carry: cubes whose upper bound improved the incumbent of their wave: their lower-bound call is still due (:856-861)
     std::vector<InnerProb> reqs; std::vector<InnerOut> outs;
     const int W = std::max(1, h->wave_nodes);
     for (;;) {
         items.clear(); items.swap(carry);
+        if (items.empty() && !S.q.empty() && (r.optError - S.q.front().lb) > SSE && S.q.front().lb >= cutoff) {
+            trace_end(r, END_CUTOFF, S.q.front().lb, SSE, cutoff);
+            r.cnt[3]++;   // the pop that meets the cutoff counts, as in the exact order
+            break;
+        }
         int popped = 0;
         while (!S.q.empty() && popped < W && (r.optError - S.q.front().lb) > SSE) {
             const RNode par = rheap_pop(S.q); r.cnt[3]++; popped++;
@@ -342,7 +350,7 @@ static goicp_status register_relaxed(Eng* h, WaveCtx& c, const BnbCfg& cfg, int 
         }
         if (items.empty()) {
             const bool empty = S.q.empty();
-            trace_end(r.trace, empty, r.optError, empty ? S.lastLb : S.q.front().lb, SSE);
+            trace_end(r, empty ? END_QUEUE_EMPTY : END_THRESHOLD, empty ? S.lastLb : S.q.front().lb, SSE, cutoff);
             if (!empty) r.cnt[3]++;   // the pop that meets the certificate counts, as in the exact order
             break;
         }
@@ -459,6 +467,7 @@ static goicp_status register_resident(Eng* h, const BnbCfg& cfg) {
     A.icp = h->sIcp.as<IcpState>(); A.outs = h->sOuts.as<PairOut>();
     A.heaps = h->qHeaps.as<HeapEnt>(); A.heapCap = heapCap; A.gscratch = h->qScratch.as<float>(); A.gstride = cfg.smemFloats; A.NdP = cfg.NdP; A.NdQ = cfg.NdQ; A.useSmem = cfg.useSmem;
     A.memo = reinterpret_cast<uint4*>(h->qMemo.p); A.memoCap = memoCap; A.ctr = h->devCounters.as<DevCounters>(); A.gridOff = cfg.gridOff; A.S3p = cfg.S3p;
+    A.cutoff = h->cutoffOn ? h->dCutoff.as<float>() : nullptr;
     cudaEventRecord(h->main.ev0, h->stream);
     CU(goicp_launch_search(A, ctas, cfg.threads, cfg.smemBytes, h->exact_sums, cfg.ct, h->stream));
     cudaEventRecord(h->main.ev1, h->stream);
@@ -477,7 +486,7 @@ static goicp_status register_resident(Eng* h, const BnbCfg& cfg) {
         r.optError = o.optError; r.optComp = o.optComp;
         for (int k = 0; k < 6; k++) r.cnt[k] = o.cnt[k];
         for (int k = 0; k < o.nEvents; k++) trace_event(r.trace, o.ev[k].kind, o.ev[k].v);
-        trace_end(r.trace, o.endKind == 1, r.optError, o.endLb, h->probs[i].dev.SSEThresh);
+        trace_end(r, o.endKind, o.endLb, h->probs[i].dev.SSEThresh, h->probs[i].cutoff);
     }
     h->stats.rerunPairs = (int)redo.size();
     if (!redo.empty()) {   // a queue outgrew its per-CTA slab: re-run those pairs with the wave scheduler, which grows the slabs on demand

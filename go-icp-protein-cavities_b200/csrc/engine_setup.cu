@@ -177,6 +177,13 @@ goicp_status upload_pairdevs(Eng* h) {
     PairDev* st = h->hPairs.as<PairDev>();
     for (size_t i = 0; i < n; i++) st[i] = h->probs[i].dev;
     CU(cudaMemcpyAsync(h->dPairs.p, st, sizeof(PairDev) * n, cudaMemcpyHostToDevice, h->stream));
+    h->cutoffOn = std::any_of(h->probs.begin(), h->probs.end(), [](const Problem& P) { return P.cutoff != INFINITY; });
+    if (h->cutoffOn) {   // (the search kernel reads no cutoffs when every pair has none)
+        CU(h->dCutoff.ensure(sizeof(float) * n));
+        CU(h->hCutoff.ensure(sizeof(float) * n));
+        for (size_t i = 0; i < n; i++) h->hCutoff.as<float>()[i] = h->probs[i].cutoff;
+        CU(cudaMemcpyAsync(h->dCutoff.p, h->hCutoff.p, sizeof(float) * n, cudaMemcpyHostToDevice, h->stream));
+    }
     CU(cudaStreamSynchronize(h->stream));
     return GOICP_OK;
 }

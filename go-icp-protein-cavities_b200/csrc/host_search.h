@@ -92,6 +92,7 @@ struct SearchResult {
     float optError = 0; double optR[9] = {1, 0, 0, 0, 1, 0, 0, 0, 1}, optT[3] = {0, 0, 0}; int optComp = 0;
     long long cnt[8] = {0, 0, 0, 0, 0, 0, 0, 0};   // goicp_result.counters
     std::string trace;
+    int endKind = 0; float endLb = 0;   // how the search ended (SearchEnd; 0: it has not run) and the lower bound of its end line
 };
 
 enum TraceKind { TRACE_INIT = 0, TRACE_ICP = 1, TRACE_BNB = 2 };   // also PairOut.ev[].kind
@@ -99,10 +100,16 @@ inline void trace_event(std::string& s, int kind, float err) {
     static const char* kinds[3] = {"Init", "ICP", "BNB"};
     tracef(s, "Error*: %g (%s)\n", err, kinds[kind % 3]);
 }
-// the end of OuterBnB: queue empty (:670-677) or the certificate optError - lb <= SSEThresh (:685)
-inline void trace_end(std::string& s, bool queueEmpty, float optError, float lb, float sse) {
-    if (queueEmpty) tracef(s, "Rotation Queue Empty\nError*: %g, LB: %g\n", optError, lb);
-    else tracef(s, "Threshold reached\nError*: %g, LB: %g, epsilon: %g\n", optError, lb, sse);
+// How OuterBnB ended (also PairOut.endKind and goicp_get_search_ends): the queue ran empty (:670-677), the certificate
+// optError - lb <= SSEThresh held at a pop (:685), or a pop that :685 did not end had lb >= the pair's error cutoff.  Best-first
+// order makes lb a lower bound on every alignment not yet ruled out, and the ruled-out ones lie above the incumbent, so the
+// optimum is >= lb >= cutoff: the pair is certified above the cutoff.
+enum SearchEnd { END_QUEUE_EMPTY = 1, END_THRESHOLD = 2, END_CUTOFF = 3 };
+inline void trace_end(SearchResult& r, int kind, float lb, float sse, float cutoff) {
+    r.endKind = kind; r.endLb = lb;
+    if (kind == END_QUEUE_EMPTY) tracef(r.trace, "Rotation Queue Empty\nError*: %g, LB: %g\n", r.optError, lb);
+    else if (kind == END_THRESHOLD) tracef(r.trace, "Threshold reached\nError*: %g, LB: %g, epsilon: %g\n", r.optError, lb, sse);
+    else tracef(r.trace, "Cutoff reached\nError*: %g, LB: %g, cutoff: %g\n", r.optError, lb, cutoff);
 }
 
 // the initial error at the identity plus the regularisation terms (:601-627)

@@ -46,6 +46,7 @@ struct OwnerSh {
     int action, actOwner, actSlot, actCancel;
     int noMorePairs, lastSpawnJ, manager;
     int waited;
+    float cutoff;                // the pair's error cutoff (+inf: none): the search ends at the first pop with lb >= cutoff that :685 does not end
     // incremental look-ahead: a full walk of the queue's front is made every SearchArgs.walkEvery pops; in between only the nodes pushed since
     // the last call are attached, if their lower bound lies inside the window the last walk covered
     int walkLeft, lastTarget, nNew; float winLb; float newLb[8]; alignas(16) unsigned newKey[8][4]; float newW[8];
@@ -240,7 +241,7 @@ __device__ void finish_pair(Cta& c, int endKind) {   // lane 0
     o.optError = os.optError; o.optComp = os.optComp;
     for (int k = 0; k < 6; k++) o.cnt[k] = os.cnt[k];
     { unsigned long long now; asm volatile("mov.u64 %0, %%globaltimer;" : "=l"(now)); o.tEndMs = (float)((now - c.A.ctl->t0ns) * 1e-6); }
-    o.status = os.status; o.endKind = endKind; o.endLb = endKind == 2 ? os.par.lb : os.lastLb; o.nEvents = min(os.nEvents, SR_MAXEV);
+    o.status = os.status; o.endKind = endKind; o.endLb = endKind >= 2 ? os.par.lb : os.lastLb; o.nEvents = min(os.nEvents, SR_MAXEV);
 }
 
 // The state words of the current node's 8 children in one load, then the result records of the finished ones (two round trips to
@@ -278,7 +279,7 @@ __device__ __forceinline__ int owner_serial(Cta& c) {
             const PairDev& P = A.pairs[os.pair];
             { unsigned long long now; asm volatile("mov.u64 %0, %%globaltimer;" : "=l"(now)); A.outs[os.pair].tStartMs = (float)((now - A.ctl->t0ns) * 1e-6); }
             os.quiet = 0; os.walkLeft = 0; os.lastTarget = -1; os.nNew = 0; os.winLb = 0.f;
-            os.SSE = P.SSEThresh; os.optComp = 0; os.status = 0; os.nEvents = 0; os.heapN = 0; os.lastLb = 0.f; os.needLbOnly = 0;
+            os.SSE = P.SSEThresh; os.cutoff = A.cutoff ? A.cutoff[os.pair] : __int_as_float(0x7f800000); os.optComp = 0; os.status = 0; os.nEvents = 0; os.heapN = 0; os.lastLb = 0.f; os.needLbOnly = 0;
             for (int k = 0; k < 6; k++) os.cnt[k] = 0;
             for (int k = 0; k < 9; k++) os.optR[k] = (k % 4 == 0) ? 1.0 : 0.0;
             os.optT[0] = os.optT[1] = os.optT[2] = 0.0;
@@ -323,6 +324,7 @@ __device__ __forceinline__ int owner_serial(Cta& c) {
             os.quiet++;
             { const long long tp0 = clock64(); os.par = rq_pop(c.rq, os.heapN); atomicAdd(&A.ctl->diag[DIAG_POP_CYCLES], (unsigned long long)(clock64() - tp0)); } os.cnt[3]++;
             if ((os.optError - os.par.lb) <= os.SSE) { finish_pair(c, 2); os.phase = OW_NONE; break; }   // :685
+            if (os.par.lb >= os.cutoff) { finish_pair(c, 3); os.phase = OW_NONE; break; }               // certified above the cutoff
             {
                 const uint4 key = node_key(os.par);
                 int g = lookup_group(c, key);   // calls made ahead of time for this node?
@@ -524,12 +526,12 @@ __device__ __forceinline__ void spawn_spec(Cta& c) {
     if (fast) {
         // fast path: the window of the last full walk still stands; only the nodes pushed since then can have entered it
         const int nNew = __shfl_sync(GOICP_FULL, nNewL, 0);
-        const float winLb = os.winLb, optE = os.optError, sse = os.SSE;
+        const float winLb = os.winLb, optE = os.optError, sse = os.SSE, cut = os.cutoff;
         __syncwarp();
         bool ok = true;
         for (int q = 0; q < nNew && ok; q++) {
             const float lb = os.newLb[q];
-            if (lb > winLb || (optE - lb) <= sse) continue;
+            if (lb > winLb || (optE - lb) <= sse || lb >= cut) continue;
             const uint4 key = *reinterpret_cast<const uint4*>(os.newKey[q]);
             int g = lookup_group_w(c, key);
             if (g >= 0) continue;
@@ -593,7 +595,7 @@ __device__ __forceinline__ void spawn_spec(Cta& c) {
         }
         __syncwarp();
         const RNodeD nd = node_at(pos);
-        if ((os.optError - nd.lb) <= os.SSE) break;   // the search ends when this node is popped (:685)
+        if ((os.optError - nd.lb) <= os.SSE || nd.lb >= os.cutoff) break;   // the search ends when this node is popped (:685 or the cutoff)
         const uint4 key = node_key(nd);
         int g = lookup_group_w(c, key);
         if (g >= 0) { if (lane == 0) { os.grpStamp[g] = os.walkStamp; os.winLb = nd.lb; } __syncwarp(); continue; }   // its calls are already out

@@ -48,8 +48,8 @@ struct PairOut {         // GoICP::Register's outputs for one pair
     float optError; int optComp;
     long long cnt[6];    // InnerBnB calls, translation pops, translation sub-cubes, rotation pops, rotation cubes, ICP calls
     int status;          // 0, GOICP_SR_*
-    int endKind;         // 1 "Rotation Queue Empty", 2 "Threshold reached"
-    float endLb;
+    int endKind;         // 1 "Rotation Queue Empty", 2 "Threshold reached", 3 "Cutoff reached" (SearchArgs.cutoff)
+    float endLb;         // kind 1: the last lower bound computed; kinds 2 and 3: the lower bound of the node popped last
     int nEvents;
     float tStartMs, tEndMs;   // diagnostics: when the pair was claimed / finished, relative to the kernel's start
     struct { int kind; float v; } ev[SR_MAXEV];   // the "Error*:" trace: kind 0 Init, 1 ICP, 2 BNB
@@ -67,6 +67,8 @@ struct SearchArgs {
     SearchCtl* ctl; OwnerHdr* hdrs; SearchSlot* slots; unsigned* states; void* rq; int rqCap; IcpState* icp; PairOut* outs;
     // inner_call
     HeapEnt* heaps; int heapCap; float* gscratch; size_t gstride; int NdP, NdQ, useSmem; uint4* memo; int memoCap; DevCounters* ctr; int gridOff, S3p;
+    // goicp_set_error_cutoff, one value per pair: the search ends at the first rotation pop with lb >= cutoff that :685 does not end (nullptr: none)
+    const float* cutoff;
 };
 
 size_t goicp_search_slot_bytes();

@@ -186,6 +186,18 @@ goicp_status goicp_batch_upload_dev(goicp_handle h, const goicp_params* p, int32
  * dprop[NdAll] the colour-dictionary index of every point, info the grid geometry.  NULL skips an output. */
 goicp_status goicp_get_cells(goicp_handle h, int32_t pair, int32_t* cell_vox, int32_t* cell_start, int32_t* cell_pts, uint32_t* cmask,
                              uint8_t* mprop, uint8_t* dprop, goicp_dt_info* info);
+/* Error cutoff for screening: cutoff[i] ends problem i's search at the first rotation pop whose lower bound lb is >= cutoff[i]
+ * while the reference's own end test (optError - lb <= SSEThresh, jly_goicp.cpp:685) does not hold.  Best-first order makes lb a
+ * lower bound on the optimum there, so the pair is certified above its cutoff; it returns the incumbent, counters and "Error*:"
+ * events it held at that pop and the end line "Cutoff reached\nError*: %g, LB: %g, cutoff: %g".  A pair that is not cut returns
+ * exactly what it returns without a cutoff; +inf is no cutoff.  n must equal the number of problems the handle holds (1 after
+ * goicp_set_model / goicp_set_data, npairs after a batch upload); NULL clears every cutoff; a NaN or another n fails with
+ * GOICP_ERR_ARG.  The batch uploads and goicp_register_batch clear the cutoffs: upload, set the cutoffs, then goicp_batch_run. */
+goicp_status goicp_set_error_cutoff(goicp_handle h, const float* cutoff_or_null, int32_t n);
+/* how the search of every problem of the last register / batch run ended: kind[i] 1 rotation queue empty, 2 threshold reached
+ * (jly_goicp.cpp:685), 3 cutoff reached (goicp_set_error_cutoff); lb[i] the lower bound of its end line (kinds 2 and 3: the
+ * lower bound of the node popped last, a certified lower bound on the pair's optimum).  One entry per problem. */
+goicp_status goicp_get_search_ends(goicp_handle h, int32_t* kind, float* lb);
 /* device-event timings (ms) and launch counts of the last batch_run / register:
  * out[0] dt build, [1] initialize, [2] inner-BnB kernels, [3] ICP kernels, [4] other; launches[0..4] likewise */
 goicp_status goicp_get_timings(goicp_handle h, float* ms5, int64_t* launches5);
