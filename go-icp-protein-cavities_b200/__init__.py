@@ -66,7 +66,7 @@ ABI_SYMBOLS = [
     "goicp_dt_download", "goicp_dt_distance", "goicp_set_nd", "goicp_initialize", "goicp_get_weights", "goicp_get_maxrotdis",
     "goicp_get_thresholds", "goicp_eval_bounds", "goicp_eval_inclusion", "goicp_inner_bnb", "goicp_icp", "goicp_register", "goicp_outer_bnb", "goicp_last_trace",
     "goicp_set_options", "goicp_set_search_mode", "goicp_register_batch", "goicp_batch_upload", "goicp_batch_upload_dev", "goicp_batch_run",
-    "goicp_get_cells", "goicp_get_timings", "goicp_set_error_cutoff", "goicp_get_search_ends",
+    "goicp_get_cells", "goicp_get_timings", "goicp_test_pairdev_uploads", "goicp_set_error_cutoff", "goicp_get_search_ends",
     "goicp_set_batch_options", "goicp_get_stats", "goicp_set_frontier_sharding", "goicp_test_exchange",
     "goicp_normalize_cloud", "goicp_scale_cloud", "goicp_rescale_translation", "goicp_apply_rigid", "goicp_rmsd",
 ]
@@ -122,6 +122,7 @@ def lib():
     u8p = C.POINTER(C.c_uint8)
     L.goicp_get_cells.argtypes = [vp, C.c_int32, ip, ip, ip, C.POINTER(C.c_uint32), u8p, u8p, C.POINTER(DTInfo)]
     L.goicp_get_timings.argtypes = [vp, fp, C.POINTER(C.c_int64)]
+    L.goicp_test_pairdev_uploads.argtypes = [vp, C.POINTER(C.c_int64)]
     L.goicp_set_error_cutoff.argtypes = [vp, fp, C.c_int32]
     L.goicp_get_search_ends.argtypes = [vp, ip, fp]
     L.goicp_set_batch_options.argtypes = [vp, C.c_int32, C.c_int32]
@@ -201,6 +202,17 @@ class Engine:
         ln = (C.c_int64 * 5)()
         self.check(self.L.goicp_get_timings(self.h, ms, ln))
         return dict(ms=list(ms), launches=list(ln))
+
+    def last_trace(self):
+        """goicp_last_trace: the "Error*:" trace of problem 0 of the last register / batch_run"""
+        return self.L.goicp_last_trace(self.h).decode()
+
+    def pairdev_uploads(self):
+        """goicp_test_pairdev_uploads: copies of the per-pair parameter records to the device so far (a run with unchanged inputs
+        makes none)"""
+        n = C.c_int64()
+        self.check(self.L.goicp_test_pairdev_uploads(self.h, C.byref(n)))
+        return n.value
 
     def set_frontier_sharding(self, rank, world, device=None):
         """Shard the InnerBnB calls of every wave of ONE registration over `world` ranks (torch.distributed must be
@@ -298,14 +310,14 @@ class Engine:
     def batch_run(self):
         res = (Result * self._npairs)()
         self.check(self.L.goicp_batch_run(self.h, res))
-        return [_result_dict(r) for r in res]
+        return _result_dicts(res)
 
     def register_batch(self, params, pairs):
         arr, keep = self._descs(pairs)
         res = (Result * len(pairs))()
         self._nprobs = len(pairs)
         self.check(self.L.goicp_register_batch(self.h, C.byref(params), len(pairs), arr, res))
-        return [_result_dict(r) for r in res]
+        return _result_dicts(res)
 
     def batch_upload_tensors(self, params, model_xyz, model_offsets, data_xyz, data_offsets, model_c=None, data_c=None,
                              model_fpfh=None, data_fpfh=None, nd=None):
@@ -423,6 +435,21 @@ def _result_dict(r):
     return dict(R=np.array(r.R).reshape(3, 3), t=np.array(r.t), optError=float(np.float32(r.optError)), optComp=int(r.optComp),
                 counters=list(r.counters), seconds_dt=r.seconds_dt, seconds_register=r.seconds_register,
                 gpu_ms_dt=r.gpu_ms_dt, gpu_ms_bnb=r.gpu_ms_bnb, gpu_ms_icp=r.gpu_ms_icp, status=int(r.status))
+
+
+_RESULT_DTYPE = np.dtype(Result)   # the ctypes fields, offsets and padding of goicp_result
+
+
+def _result_dicts(res):
+    """[_result_dict(r) for r in res] for a Result array, column by column: one view of the array as a structured numpy array,
+    R and t as rows of one array each, every other column converted to Python numbers at once"""
+    a = np.frombuffer(res, dtype=_RESULT_DTYPE)
+    R = np.array(a["R"], np.float64).reshape(-1, 3, 3)
+    t = np.array(a["t"], np.float64)
+    cols = [a[k].tolist() for k in ("optError", "optComp", "counters", "seconds_dt", "seconds_register", "gpu_ms_dt", "gpu_ms_bnb", "gpu_ms_icp", "status")]
+    return [dict(R=R[i], t=t[i], optError=e, optComp=oc, counters=c, seconds_dt=sd, seconds_register=sr, gpu_ms_dt=md, gpu_ms_bnb=mb,
+                 gpu_ms_icp=mi, status=st)
+            for i, (e, oc, c, sd, sr, md, mb, mi, st) in enumerate(zip(*cols))]
 
 
 class GoICP:

@@ -80,7 +80,9 @@ goicp_status goicp_create(goicp_handle* out, int device, void* stream_or_null) {
         delete h; return fail(nullptr, GOICP_ERR_CUDA, "kernel preload failed: %s (library built for sm_100a only)", cudaGetErrorString(e));
     }
     if (h->devCounters.ensure(sizeof(DevCounters)) != cudaSuccess || cudaMemset(h->devCounters.p, 0, sizeof(DevCounters)) != cudaSuccess) { delete h; return fail(nullptr, GOICP_ERR_CUDA, "device allocation failed"); }
-    if (h->main.init(false, h->stream) != GOICP_OK) { delete h; return fail(nullptr, GOICP_ERR_CUDA, "event creation failed"); }
+    if (h->main.init(false, h->stream) != GOICP_OK || cudaEventCreateWithFlags(&h->evPairs, cudaEventDisableTiming) != cudaSuccess) {
+        goicp_destroy(h); return fail(nullptr, GOICP_ERR_CUDA, "event creation failed");
+    }
     goicp_params_default(&h->params); h->haveParams = true;
     *out = h;
     return GOICP_OK;
@@ -95,6 +97,7 @@ void goicp_destroy(goicp_handle h) {
     h->hStage.release(); h->hPairs.release(); h->hPrep.release(); h->hOuts.release(); h->hCutoff.release(); h->qHeaps.release(); h->qScratch.release(); h->qMemo.release(); h->devCounters.release();
     h->main.release();
     for (auto& w : h->workers) w->release();
+    if (h->evPairs) cudaEventDestroy(h->evPairs);
     if (h->ownStream) cudaStreamDestroy(h->stream);
     delete h;
 }
@@ -121,7 +124,7 @@ goicp_status goicp_set_params(goicp_handle h, const goicp_params* p) {
                              (p->trimFraction < 0.001) != (h->params.trimFraction < 0.001) ||
                              p->cfpfh != h->params.cfpfh || p->regularizationFPFH != h->params.regularizationFPFH ||
                              (p->regularizationNeighbors > 0) != (h->params.regularizationNeighbors > 0);   // every key K1 or the arena layout depends on
-    h->params = *p; h->haveParams = true;
+    h->params = *p; h->haveParams = true; h->pairsDirty = true;
     for (auto& P : h->probs) { P.initialized = false; if (gridChanged) P.prepared = P.dt_built = false; }
     return GOICP_OK;
 }
@@ -140,7 +143,7 @@ static goicp_status build_dt_impl(goicp_handle h, goicp_dt_info* out, bool repla
     if (P.Nm < 1 || P.NdAll < 1) return fail(h, GOICP_ERR_ARG, "build_dt: model and data clouds must be set first");
     cudaSetDevice(h->device);
     if ((s = prepare_all(h))) return s;
-    if ((s = build_dt_all(h, replay))) return s;
+    if ((s = build_dt_all(h, replay, true))) return s;
     h->dtUploaded = false;
     if (out) *out = P.info;
     return GOICP_OK;
@@ -213,14 +216,16 @@ goicp_status goicp_set_nd(goicp_handle h, int32_t nd) {
     goicp_status s; if ((s = ensure_single(h))) return s;
     Problem& P = h->probs[0];
     if (nd < 1 || nd > P.NdAll) return fail(h, GOICP_ERR_ARG, "set_nd: %d outside [1,%d]", nd, P.NdAll);
-    P.Nd = nd; P.initialized = false;
+    P.Nd = nd; P.initialized = false; h->pairsDirty = true;
     return GOICP_OK;
 }
 goicp_status goicp_initialize(goicp_handle h) {
     if (!h) return GOICP_ERR_ARG;
     goicp_status s; if ((s = ensure_single(h))) return s;
     cudaSetDevice(h->device);
-    return initialize_all(h);
+    if ((s = initialize_all(h))) return s;
+    h->main.collect(1);
+    return GOICP_OK;
 }
 goicp_status goicp_get_weights(goicp_handle h, float* w) {
     if (!h || !w) return GOICP_ERR_ARG;
@@ -272,6 +277,7 @@ goicp_status goicp_eval_bounds(goicp_handle h, const float* R, const int32_t* le
     if (incomp_minmax) CU(cudaMemcpyAsync(incomp_minmax, dI, sizeof(int) * 2 * nt, cudaMemcpyDeviceToHost, h->stream));
     if (fpfh_minmax) CU(cudaMemcpyAsync(fpfh_minmax, dFm, sizeof(int) * 2 * nt, cudaMemcpyDeviceToHost, h->stream));
     CU(cudaStreamSynchronize(h->stream));
+    h->main.collect(2);
     return GOICP_OK;
 }
 
@@ -427,7 +433,8 @@ goicp_status goicp_batch_run(goicp_handle h, goicp_result* results) {
     cudaSetDevice(h->device);
     h->main.reset_timing();
     goicp_status s;
-    if ((s = build_dt_all(h, h->use_dt_replay && h->params.distTransSize <= 32))) return s;
+    // DT, Initialize and the search are enqueued back to back; the host waits once, for the search
+    if ((s = build_dt_all(h, h->use_dt_replay && h->params.distTransSize <= 32, false))) return s;
     if ((s = register_all(h))) return s;
     for (size_t i = 0; i < h->probs.size(); i++) fill_result(h, h->probs[i], results + i);
     h->trace = h->probs[0].res.trace;
@@ -460,6 +467,7 @@ goicp_status goicp_set_error_cutoff(goicp_handle h, const float* cutoff_or_null,
     if (cutoff_or_null)
         for (int i = 0; i < n; i++) if (std::isnan(cutoff_or_null[i])) return fail(h, GOICP_ERR_ARG, "set_error_cutoff: the cutoff of problem %d is NaN", i);
     for (int i = 0; i < n; i++) h->probs[i].cutoff = cutoff_or_null ? cutoff_or_null[i] : INFINITY;
+    h->pairsDirty = true;
     return GOICP_OK;
 }
 goicp_status goicp_get_search_ends(goicp_handle h, int32_t* kind, float* lb) {
@@ -479,6 +487,11 @@ goicp_status goicp_set_batch_options(goicp_handle h, int32_t groups, int32_t slo
 goicp_status goicp_get_stats(goicp_handle h, double* out16) {
     if (!h || !out16) return GOICP_ERR_ARG;
     memcpy(out16, &h->stats, sizeof h->stats);
+    return GOICP_OK;
+}
+goicp_status goicp_test_pairdev_uploads(goicp_handle h, int64_t* count) {
+    if (!h || !count) return GOICP_ERR_ARG;
+    *count = h->pairUploads;
     return GOICP_OK;
 }
 goicp_status goicp_get_timings(goicp_handle h, float* ms5, int64_t* launches5) {

@@ -113,6 +113,8 @@ struct WaveCtx {
     bool counterReady = false;
     cudaEvent_t ev0 = nullptr, ev1 = nullptr, evDone = nullptr;
     float ms[5] = {0, 0, 0, 0, 0}; long long launches[5] = {0, 0, 0, 0, 0};
+    cudaEvent_t tev[5][2] = {};                  // EvTimer: start / end of the last timed group of each slot
+    bool tPending[5] = {}; int tLaunches[5] = {};   // ... recorded, not yet added to ms / launches (collect)
     long long waves = 0, callsLaunched = 0;
     double tLogic = 0, tInnerEnq = 0, tInnerWait = 0;   // host seconds
     int heapCap = 1 << 14;
@@ -122,7 +124,18 @@ struct WaveCtx {
         if (own && cudaStreamCreateWithFlags(&stream, cudaStreamNonBlocking) != cudaSuccess) return GOICP_ERR_CUDA;
         if (cudaEventCreate(&ev0) != cudaSuccess || cudaEventCreate(&ev1) != cudaSuccess ||
             cudaEventCreateWithFlags(&evDone, cudaEventBlockingSync | cudaEventDisableTiming) != cudaSuccess) return GOICP_ERR_CUDA;
+        for (auto& t : tev) if (cudaEventCreate(&t[0]) != cudaSuccess || cudaEventCreate(&t[1]) != cudaSuccess) return GOICP_ERR_CUDA;
         return GOICP_OK;
+    }
+    // adds the pending EvTimer groups (every slot, or `slot` only) to ms / launches, waiting for their end events; after the
+    // stream has been synchronised past them this does not wait
+    void collect(int slot = -1) {
+        for (int k = 0; k < 5; k++) {
+            if (!tPending[k] || (slot >= 0 && k != slot)) continue;
+            float t = 0;
+            cudaEventSynchronize(tev[k][1]); cudaEventElapsedTime(&t, tev[k][0], tev[k][1]);
+            ms[k] += t; launches[k] += tLaunches[k]; tPending[k] = false;
+        }
     }
     // waits without spinning a host core (worker threads outnumber cores)
     cudaError_t sync() {
@@ -130,7 +143,7 @@ struct WaveCtx {
         return cudaEventSynchronize(evDone);
     }
     void reset_timing() {
-        memset(ms, 0, sizeof ms); memset(launches, 0, sizeof launches); waves = callsLaunched = 0;
+        memset(ms, 0, sizeof ms); memset(launches, 0, sizeof launches); memset(tPending, 0, sizeof tPending); waves = callsLaunched = 0;
         tLogic = tInnerEnq = tInnerWait = 0;
     }
     void release() {
@@ -139,6 +152,7 @@ struct WaveCtx {
         mProbs.release(); mOuts.release(); mIcp.release();
         if (ev0) cudaEventDestroy(ev0); if (ev1) cudaEventDestroy(ev1); if (evDone) cudaEventDestroy(evDone);
         ev0 = ev1 = evDone = nullptr;
+        for (auto& t : tev) for (cudaEvent_t& e : t) { if (e) cudaEventDestroy(e); e = nullptr; }
         if (ownStream && stream) cudaStreamDestroy(stream);
         stream = nullptr;
     }
@@ -170,6 +184,9 @@ struct goicp_handle_s {
     DevBuf qHeaps, qScratch, qMemo, devCounters;   // per-CTA slabs of the device-resident search: translation queues, staging arrays (large Nd), corner memo; DevCounters
     DevBuf sCtl, sHdrs, sSlots, sStates, sRq, sIcp, sOuts; PinBuf hOuts;   // device-resident search (k_search.cu)
     DevBuf dCutoff; PinBuf hCutoff; bool cutoffOn = false;   // Problem::cutoff of every pair, uploaded by upload_pairdevs when one is finite
+    // upload_pairdevs: dPairs / dCutoff are stale (set by everything the PairDev fields or the cutoffs derive from: parameters,
+    // Nd, the clouds' layout, the cutoffs); evPairs follows the last copy out of hPairs / hCutoff; uploads counts the copies
+    bool pairsDirty = true; cudaEvent_t evPairs = nullptr; long long pairUploads = 0;
     int spec_groups = SR_NGROUP - 4;   // device-resident search: most rotation-queue nodes with speculative calls per owner CTA (0: never speculate)
     int shardRank = 0, shardN = 1; goicp_allgather_fn allgather = nullptr; void* allgatherUser = nullptr;   // frontier sharding
     std::vector<InnerOut> xSend, xRecv;
@@ -177,7 +194,8 @@ struct goicp_handle_s {
     int resident = 1;            // 1: device-resident search (k_search.cu) whenever the clouds allow it; 0: wave scheduler (one launch per wave, host-side OuterBnB)
     std::vector<std::unique_ptr<WaveCtx>> workers;
     std::mutex errMutex;
-    std::string err, trace;
+    std::string err;
+    Trace trace;   // of problem 0 after the last register or batch run; goicp_last_trace formats it
     SearchStats stats;
 };
 
@@ -193,10 +211,12 @@ inline goicp_status fail(Eng* h, goicp_status s, const char* fmt, ...) {
 
 inline size_t al256(size_t b) { return (b + 255) & ~(size_t)255; }
 
-struct EvTimer {   // CUDA-event time of a kernel group on a wave context's stream
+// CUDA-event time of a kernel group on a wave context's stream.  The events are recorded without waiting for them;
+// WaveCtx::collect adds the time to ms[slot], so that phases can be enqueued back to back and read after one synchronise.
+struct EvTimer {
     WaveCtx& c; int slot;
-    EvTimer(WaveCtx& c_, int slot_) : c(c_), slot(slot_) { cudaEventRecord(c.ev0, c.stream); }
-    void stop(int nlaunch) { cudaEventRecord(c.ev1, c.stream); cudaEventSynchronize(c.ev1); float ms = 0; cudaEventElapsedTime(&ms, c.ev0, c.ev1); c.ms[slot] += ms; c.launches[slot] += nlaunch; }
+    EvTimer(WaveCtx& c_, int slot_) : c(c_), slot(slot_) { c.collect(slot); cudaEventRecord(c.tev[slot][0], c.stream); }
+    void stop(int nlaunch) { cudaEventRecord(c.tev[slot][1], c.stream); c.tPending[slot] = true; c.tLaunches[slot] = nlaunch; }
 };
 
 // keys of the trimmed-ICP bitonic sort (icp_device.cuh): next power of two >= n, at least 32
@@ -206,7 +226,7 @@ struct BnbCfg { int NdP, NdQ; size_t smemFloats, smemBytes; int useSmem, perSM, 
 // engine_setup.cu
 goicp_status upload_clouds(Eng* h, const goicp_pair_desc* src, bool onDevice);
 goicp_status upload_pairdevs(Eng* h);
-goicp_status build_dt_all(Eng* h, bool replay);
+goicp_status build_dt_all(Eng* h, bool replay, bool wait);   // wait: until the DT is built (its timing is then in main.ms[0])
 goicp_status initialize_all(Eng* h);
 BnbCfg bnb_config(Eng* h);
 goicp_status prepare_all(Eng* h);

@@ -485,7 +485,8 @@ static goicp_status register_resident(Eng* h, const BnbCfg& cfg) {
         memcpy(r.optR, o.R, sizeof r.optR); memcpy(r.optT, o.t, sizeof r.optT);
         r.optError = o.optError; r.optComp = o.optComp;
         for (int k = 0; k < 6; k++) r.cnt[k] = o.cnt[k];
-        for (int k = 0; k < o.nEvents; k++) trace_event(r.trace, o.ev[k].kind, o.ev[k].v);
+        r.trace.events.resize(o.nEvents);
+        for (int k = 0; k < o.nEvents; k++) r.trace.events[k] = TraceEvent{o.ev[k].kind, o.ev[k].v};
         trace_end(r, o.endKind, o.endLb, h->probs[i].dev.SSEThresh, h->probs[i].cutoff);
     }
     h->stats.rerunPairs = (int)redo.size();
@@ -560,6 +561,7 @@ goicp_status register_all(Eng* h) {
             h->main.tLogic += w->tLogic; h->main.tInnerEnq += w->tInnerEnq; h->main.tInnerWait += w->tInnerWait;
         }
     }
+    h->main.collect();   // the DT / Initialize timers (every scheduler has synchronised the handle's stream past them)
     const double dt = secs_since(t0);
     for (auto& P : h->probs) P.t_reg = dt / std::max(1, np);
     SearchStats& st = h->stats;

@@ -67,6 +67,7 @@ goicp_status upload_clouds(Eng* h, const goicp_pair_desc* src, bool onDevice) {
     });
     if (!onDevice) CU(cudaMemcpyAsync(h->dRaw.p, h->hStage.p, rawTot, cudaMemcpyHostToDevice, h->stream));
     h->packElems = maxElems;
+    h->pairsDirty = true;
     for (auto& P : h->probs) { P.uploaded = true; P.prepared = P.dt_built = P.initialized = false; }
     return GOICP_OK;
 }
@@ -120,11 +121,16 @@ static goicp_status layout_work(Eng* h, bool ncellsBound) {
         D.g.S = S; D.g.ncells = nc; D.g.xMin = P.info.xMin; D.g.yMin = P.info.yMin; D.g.zMin = P.info.zMin; D.g.scale = P.info.scale;
         D.Nm = P.Nm; D.Nd = P.Nd; D.NdAll = P.NdAll;
     }
+    h->pairsDirty = true;
     return GOICP_OK;
 }
 
-// fills the parameter-derived fields of every PairDev (GoICP::Initialize :180-267 scalars) and uploads the array
+// fills the parameter-derived fields of every PairDev (GoICP::Initialize :180-267 scalars) and uploads the array, with the
+// cutoffs; nothing to do unless something they derive from changed since the last upload (Eng::pairsDirty).  The copies are
+// stream-ordered before every kernel that reads them; the host only waits for the previous copy before it rewrites the pinned
+// staging buffers.
 goicp_status upload_pairdevs(Eng* h) {
+    if (!h->pairsDirty) return GOICP_OK;
     const goicp_params& p = h->params;
     const bool doTrim = !(p.trimFraction < 0.001);   // GoICP() :54 sets true; readConfig clears it (jly_main.cpp:259)
     for (auto& P : h->probs) {
@@ -172,6 +178,7 @@ goicp_status upload_pairdevs(Eng* h) {
         }
     }
     const size_t n = h->probs.size();
+    CU(cudaEventSynchronize(h->evPairs));   // (returns at once when the previous copy is done, or there was none)
     CU(h->dPairs.ensure(sizeof(PairDev) * n));
     CU(h->hPairs.ensure(sizeof(PairDev) * n));
     PairDev* st = h->hPairs.as<PairDev>();
@@ -184,11 +191,12 @@ goicp_status upload_pairdevs(Eng* h) {
         for (size_t i = 0; i < n; i++) h->hCutoff.as<float>()[i] = h->probs[i].cutoff;
         CU(cudaMemcpyAsync(h->dCutoff.p, h->hCutoff.p, sizeof(float) * n, cudaMemcpyHostToDevice, h->stream));
     }
-    CU(cudaStreamSynchronize(h->stream));
+    CU(cudaEventRecord(h->evPairs, h->stream));
+    h->pairsDirty = false; h->pairUploads++;
     return GOICP_OK;
 }
 
-goicp_status build_dt_all(Eng* h, bool replay) {
+goicp_status build_dt_all(Eng* h, bool replay, bool wait) {
     const int S = h->params.distTransSize;
     auto t0 = clk::now();
     goicp_status s = upload_pairdevs(h);
@@ -208,6 +216,7 @@ goicp_status build_dt_all(Eng* h, bool replay) {
     }
     tm.stop(nl);
     CU(cudaGetLastError());
+    if (wait) h->main.collect(0);
     const double dt = secs_since(t0) / std::max<size_t>(1, h->probs.size());
     for (auto& P : h->probs) { P.dt_built = true; P.t_dt = dt; }
     return GOICP_OK;

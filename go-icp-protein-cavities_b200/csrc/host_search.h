@@ -87,29 +87,46 @@ inline RNode child_of(const RNode& par, int j) {
     return nr;
 }
 
-// What GoICP::Register leaves behind for one pair (GoICP::Initialize :240-241 resets optR / optT).
-struct SearchResult {
-    float optError = 0; double optR[9] = {1, 0, 0, 0, 1, 0, 0, 0, 1}, optT[3] = {0, 0, 0}; int optComp = 0;
-    long long cnt[8] = {0, 0, 0, 0, 0, 0, 0, 0};   // goicp_result.counters
-    std::string trace;
-    int endKind = 0; float endLb = 0;   // how the search ended (SearchEnd; 0: it has not run) and the lower bound of its end line
-};
-
 enum TraceKind { TRACE_INIT = 0, TRACE_ICP = 1, TRACE_BNB = 2 };   // also PairOut.ev[].kind
-inline void trace_event(std::string& s, int kind, float err) {
-    static const char* kinds[3] = {"Init", "ICP", "BNB"};
-    tracef(s, "Error*: %g (%s)\n", err, kinds[kind % 3]);
-}
 // How OuterBnB ended (also PairOut.endKind and goicp_get_search_ends): the queue ran empty (:670-677), the certificate
 // optError - lb <= SSEThresh held at a pop (:685), or a pop that :685 did not end had lb >= the pair's error cutoff.  Best-first
 // order makes lb a lower bound on every alignment not yet ruled out, and the ruled-out ones lie above the incumbent, so the
 // optimum is >= lb >= cutoff: the pair is certified above the cutoff.
 enum SearchEnd { END_QUEUE_EMPTY = 1, END_THRESHOLD = 2, END_CUTOFF = 3 };
+
+// The "Error*:" trace OuterBnB prints (jly_goicp.cpp:627-839, :670-685), kept as the values it is printed from: the improvement
+// events in order and the end record.  A batch records every pair's trace but reads at most one, so the text is only built by
+// str() / c_str(), when it is read.
+struct TraceEvent { int kind; float v; };   // TraceKind, the new incumbent
+struct Trace {
+    std::vector<TraceEvent> events;
+    int endKind = 0; float endErr = 0, endLb = 0, endSse = 0, endCutoff = 0;   // SearchEnd (0: no end line yet) and what it prints
+    mutable std::string text;   // the last str()
+    const std::string& str() const {
+        static const char* kinds[3] = {"Init", "ICP", "BNB"};
+        text.clear();
+        for (const TraceEvent& e : events) tracef(text, "Error*: %g (%s)\n", e.v, kinds[e.kind % 3]);
+        if (endKind == END_QUEUE_EMPTY) tracef(text, "Rotation Queue Empty\nError*: %g, LB: %g\n", endErr, endLb);
+        else if (endKind == END_THRESHOLD) tracef(text, "Threshold reached\nError*: %g, LB: %g, epsilon: %g\n", endErr, endLb, endSse);
+        else if (endKind != 0) tracef(text, "Cutoff reached\nError*: %g, LB: %g, cutoff: %g\n", endErr, endLb, endCutoff);
+        return text;
+    }
+    const char* c_str() const { return str().c_str(); }
+};
+
+// What GoICP::Register leaves behind for one pair (GoICP::Initialize :240-241 resets optR / optT).
+struct SearchResult {
+    float optError = 0; double optR[9] = {1, 0, 0, 0, 1, 0, 0, 0, 1}, optT[3] = {0, 0, 0}; int optComp = 0;
+    long long cnt[8] = {0, 0, 0, 0, 0, 0, 0, 0};   // goicp_result.counters
+    Trace trace;
+    int endKind = 0; float endLb = 0;   // how the search ended (SearchEnd; 0: it has not run) and the lower bound of its end line
+};
+
+inline void trace_event(Trace& t, int kind, float err) { t.events.push_back(TraceEvent{kind, err}); }
 inline void trace_end(SearchResult& r, int kind, float lb, float sse, float cutoff) {
     r.endKind = kind; r.endLb = lb;
-    if (kind == END_QUEUE_EMPTY) tracef(r.trace, "Rotation Queue Empty\nError*: %g, LB: %g\n", r.optError, lb);
-    else if (kind == END_THRESHOLD) tracef(r.trace, "Threshold reached\nError*: %g, LB: %g, epsilon: %g\n", r.optError, lb, sse);
-    else tracef(r.trace, "Cutoff reached\nError*: %g, LB: %g, cutoff: %g\n", r.optError, lb, cutoff);
+    Trace& t = r.trace;
+    t.endKind = kind; t.endErr = r.optError; t.endLb = lb; t.endSse = sse; t.endCutoff = cutoff;
 }
 
 // the initial error at the identity plus the regularisation terms (:601-627)

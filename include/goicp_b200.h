@@ -201,6 +201,9 @@ goicp_status goicp_get_search_ends(goicp_handle h, int32_t* kind, float* lb);
 /* device-event timings (ms) and launch counts of the last batch_run / register:
  * out[0] dt build, [1] initialize, [2] inner-BnB kernels, [3] ICP kernels, [4] other; launches[0..4] likewise */
 goicp_status goicp_get_timings(goicp_handle h, float* ms5, int64_t* launches5);
+/* test hook: how many times the handle has copied its per-pair parameter records to the device.  A register or batch run copies
+ * them only when something they derive from changed since the last copy (parameters, Nd, clouds, error cutoffs). */
+goicp_status goicp_test_pairdev_uploads(goicp_handle h, int64_t* count);
 /* wave scheduler only (large clouds, frontier sharding, GOICP_PERSISTENT=0): `groups` worker streams (0 = auto), each advancing
  * `slots` pairs (0 = auto) in lock-step waves and pulling the next pair from a shared counter when one finishes.  The default
  * device-resident search needs no host threads (bo1_GoICP.py:40-54 is one serial process per pair). */
