@@ -10,7 +10,11 @@ an L2 flush and one `batch_run` between two CUDA events on the engine's stream. 
   - dt / initialize / search: the library's own event timings of the three phases (goicp_get_timings), mean per step;
   - gap: ms_per_step - (dt + initialize + search), the step time in which none of the three phases runs: host work, copies and
     the GPU waiting for the host;
-  - host_ms: the host wall time of the step's batch_run call.
+  - host_ms: the host wall time of the step's batch_run call;
+  - calls_executed / calls_used / cycles_per_pop: InnerBnB calls the search kernel ran and those the reference's order consumed,
+    and CTA-cycles per translation pop inside calls (Engine.stats of the last step).
+With GOICP_DEBUG set (in the environment or with @GOICP_DEBUG=1) the library's per-step search report of each run is printed
+too; a tree built with `make EXTRA=-DGOICP_PHASE_TIMING` adds the cycles per pop of each phase to it.
 It prints the GPU's name and power limit first and a summary of min / median / max per tree last."""
 import argparse
 import json
@@ -57,8 +61,10 @@ def worker(tree, steps, warmup, npairs):
     torch.cuda.synchronize(dev)
     step = sum(a.elapsed_time(b) for a, b in ev) / steps
     dt, ini, search = (p / steps for p in phase)
+    st = eng.stats()
     row = dict(tree=tree, env=os.environ.get("STEP_OVERHEAD_ENV", ""), pairs=npairs, steps=steps, ms_per_step=step, dt=dt, initialize=ini, search=search,
-               gap=step - (dt + ini + search), host_ms=1e3 * host / steps)
+               gap=step - (dt + ini + search), host_ms=1e3 * host / steps, calls_executed=st["calls_executed"], calls_used=st["calls_used"],
+               cycles_per_pop=st.get("search_kernel", {}).get("cycles_per_pop_in_calls"))
     print("ROW " + json.dumps(row), flush=True)
 
 
@@ -88,6 +94,8 @@ def main():
             if out.returncode != 0 or not line:
                 print(out.stdout[-2000:], out.stderr[-4000:])
                 raise SystemExit(f"worker failed on {spec}")
+            if "GOICP_DEBUG" in {**os.environ, **env}:
+                print(out.stderr, end="", flush=True)
             row = json.loads(line[0][4:]); row["round"] = r; row["leg"] = spec
             print(json.dumps({k: round(v, 2) if isinstance(v, float) else v for k, v in row.items()}), flush=True)
             rows.append(row)
